@@ -2,6 +2,7 @@
 """Benchmark of the EgoT2 task-translation hot path on B200 (contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dtype bf16|fp32]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): translator forward+backward clips/sec.  Default workload = BASELINE config 2:
 HHI TaskFusionMFTransformer3Task (LAM+TTM+ASD -> TTM) training, 1 layer, hidden 128, 4 heads, FFN 2048,
@@ -10,14 +11,24 @@ One step = forward + fused weighted-CE loss + backward of every translator param
 all-reduce of the flat gradient arena) + one fused Adam launch.
 
 Lines printed by rank 0 (ONE JSON line):
-  value     whole-job clips/s, features already resident in HBM (rotating pool larger than L2), CUDA-event timed,
-            max over ranks;
+  value     whole-job clips/s over exactly K timed steps, features already resident in HBM (rotating pool larger than L2),
+            CUDA-event timed, max over ranks; at the default K = 2000 that window lasts about 0.66 s (0.33 ms steps on one
+            B200 at 1000 W), while K = 20 gives a window of a few milliseconds.  Only this figure follows --steps exactly:
+            e2e, fwd_only, fp32, module_path and the other workloads each time their own count, derived from K but clamped;
   e2e       same step driven from pinned HOST buffers through TranslatorTrainer.train_stream_host: every step's H2D copy of
             features+labels and D2H read of its loss are inside the timed region (double-buffered on a copy stream);
   roofline  the dominant kernel of the step (largest share of the summed kernel time), timed by CUDA events that the
             library records around each launch on the launch stream during a pass of eager steps after the timed region;
   cpu_baseline  the CPU oracle (torch restatement of the reference translator) on this box's host cores.
 `--impl reference` times that CPU implementation as the reference arm.
+
+--dump-outputs DIR: after the K timed steps, rank 0 writes what the last of them computed - the loss it returned
+(loss.npy) and, where the step runs from a CUDA graph of the single-model trainer, the translator output it computed
+(logits.npy) - in float32, so that two builds run with the same arguments (same seeded weights and inputs) can be compared
+output for output.  The updated parameters are deliberately not written: the kernels' reductions add partial sums in no
+fixed order, and Adam turns those last-bit differences into whole learning-rate steps wherever a gradient is rounding
+noise (the attention key bias has an exactly zero gradient), so the parameters differ between two runs of one build by
+far more than rounding, while what the step computes from them does not.
 """
 from __future__ import annotations
 
@@ -54,6 +65,23 @@ WORKLOADS = {
                         g_kind="hoi", g_batches=dict(pnr=32, oscc=32, action=32)),
 }
 L2_BYTES = 126 * 2 ** 20
+DUMP_BYTES = 60 * 2 ** 20         # array payload of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: tensor} as out_dir/<name>.npy in float32.  When all of them together exceed DUMP_BYTES, every tensor is
+    replaced by the same fraction of its elements (at least one), picked by a fixed seed (flattened, in index order), so
+    that two runs sample identical positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keep = min(1.0, (DUMP_BYTES // 4 - len(arrays)) / sum(t.numel() for t in arrays.values()))
+    g = torch.Generator().manual_seed(0)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if keep < 1.0:
+            flat = a.reshape(-1)
+            a = flat[torch.randperm(flat.numel(), generator=g)[:max(1, int(flat.numel() * keep))].sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def load_peaks():
@@ -388,7 +416,7 @@ def other_workload_line(name, dev, rank, world, steps, warmup, batch=0):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=2000)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="hhi_ttm3_train_b256", choices=sorted(WORKLOADS))
@@ -398,6 +426,8 @@ def main():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extras", action="store_true", help="headline line only (A/B runs): no fwd_only / fp32 / "
                     "module_path / gpu_baseline / other workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss and translator output "
+                    "as DIR/<name>.npy (float32, under 64 MB in all)")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
     if args.batch:
@@ -428,16 +458,17 @@ def main():
             torch.distributed.barrier()
         torch.cuda.synchronize(dev)
 
-    # ---- device-resident throughput (the contract's K steps) ...
+    # ---- device-resident throughput over the K timed steps
     clocks = ClockSampler(local_rank)
     tr = build_trainer(args.workload, wl, spec, dev, args.dtype, not args.no_graphs)
     pool, feat_bytes = build_pool(wl, spec, B, dev, args.dtype, rank)
     n_pool = len(pool)
+    last = []            # (loss, graph key) of the latest step
 
     def run_steps(n, start=0):
         for i in range(n):
             fe, la = pool[(start + i) % n_pool]
-            tr.train_step(fe, la, graph_key=(start + i) % n_pool)
+            last[:] = [tr.train_step(fe, la, graph_key=(start + i) % n_pool), (start + i) % n_pool]
 
     run_steps(max(args.warmup, n_pool if tr.use_graphs else args.warmup))     # capture every pool graph first
     barrier()
@@ -449,13 +480,21 @@ def main():
     barrier()
     if rank == 0:
         clocks.start()
-    ms_total = timed(lambda i: run_steps(1, start=1 + i), args.steps, dev, world)
-    # ... and a sustained region of >= 0.5 s (the K-step region is a few ms at the driver's K), reported beside it
-    sus_steps = max(args.steps, int(0.6 / max(ms_total / args.steps * 1e-3, 1e-6)))
-    sus_steps = min(sus_steps, 20000)
-    ms_sus = timed(lambda i: run_steps(1, start=7 + i), sus_steps, dev, world)
-    clock_info = clocks.stop() if rank == 0 else None
+    try:
+        ms_total = timed(lambda i: run_steps(1, start=1 + i), args.steps, dev, world)
+    finally:
+        clock_info = clocks.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the step's buffers are overwritten by the legs below: copied out before any of them runs
+        from egot2_b200.engine import Activations
+        from egot2_b200.trainer import TranslatorTrainer
+        outputs = {"loss": last[0].reshape(1)}
+        if isinstance(tr, TranslatorTrainer) and tr.use_graphs:
+            act = tr._graphs[last[1]][-1]          # the graph cache entry ends with the activations its replays write
+            assert isinstance(act, Activations), f"unexpected graph cache entry {type(act)}: no logits to dump"
+            outputs["logits"] = act.t["out"]
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- end-to-end from pinned host buffers (H2D + step + D2H of the loss inside the timed region)
     host = []
@@ -554,8 +593,6 @@ def main():
         "step_roofline": {"bound": "tensor", "achieved": tfs / world, "peak": peaks["bf16_tflops_sustained"], "unit": "TFLOP/s",
                           "frac": tfs / world / peaks["bf16_tflops_sustained"],
                           "note": "whole step, per GPU: SURVEY 8(d) FLOPs_fwd+bwd per clip x clips / step time"},
-        "sustained": {"steps": sus_steps, "ms_per_step": ms_sus / sus_steps, "value": world * B * sus_steps / (ms_sus * 1e-3),
-                      "note": "same step, timed region >= 0.5 s"},
         "clocks": clock_info,
         "e2e": {"value": e2e_value, "unit": "clips/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": 4,
                 "steps": e2e_steps, "h2d_copy_alone_ms": h2d_ms, "h2d_copy_alone_gbs": h2d_gbs,

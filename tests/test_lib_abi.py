@@ -71,10 +71,15 @@ def test_struct_layouts_match_header(built):
 
 
 def test_no_fallback_without_cuda():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
-    from egot2_b200 import _lib, specs
-    from egot2_b200.engine import TranslatorEngine
-    with pytest.raises(_lib.Egot2Error):
-        TranslatorEngine(specs.hhi_ttm_spec(), "cpu")
+    """Without a CUDA device the engine refuses to run; checked in a child process that sees no device, so that a machine
+    with a GPU checks it too."""
+    import subprocess
+    import sys
+    code = ("import pytest, torch\n"
+            "from egot2_b200 import _lib, specs\n"
+            "from egot2_b200.engine import TranslatorEngine\n"
+            "assert not torch.cuda.is_available()\n"
+            "with pytest.raises(_lib.Egot2Error):\n"
+            "    TranslatorEngine(specs.hhi_ttm_spec(), 'cpu')\n")
+    flags = ["-s"] if sys.flags.no_user_site else []
+    subprocess.run([sys.executable, *flags, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), check=True)

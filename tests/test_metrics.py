@@ -1,14 +1,11 @@
 """On-device PNR / OSCC metrics (egot2_b200/metrics.py -> egot2_pnr_metrics) against the CPU restatement, and the
-restatement against the reference's own functions (HOI/evaluation/pnr/metrics.py) where the reference tree exists."""
-import importlib.util
-import os
+restatement against the reference's own functions (HOI/evaluation/pnr/metrics.py) where oracle/ref_shims finds them."""
+import importlib
 
 import pytest
 import torch
 
 from oracle import metrics_oracle as MO
-
-REF = "/root/reference/HOI/evaluation/pnr/metrics.py"
 
 
 def _inputs(B, seed, ties=False):
@@ -29,7 +26,7 @@ def _inputs(B, seed, ties=False):
     return preds, labels, sc, fps, info, oscc_pred, oscc_lab
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present")
+@pytest.mark.requires_reference
 @pytest.mark.parametrize("B,seed,ties", [(1, 0, False), (37, 1, False), (256, 2, True)])
 def test_oracle_matches_reference_metrics(B, seed, ties):
     import sys
@@ -42,9 +39,8 @@ def test_oracle_matches_reference_metrics(B, seed, ties):
                 stub = types.ModuleType(name)
                 stub.Metric = object
                 sys.modules[name] = stub
-    spec = importlib.util.spec_from_file_location("ref_pnr_metrics", REF)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    from oracle import ref_shims
+    ref = ref_shims._load_file("ref_pnr_metrics", "HOI/evaluation/pnr/metrics.py")
     preds, labels, sc, fps, info, op, ol = _inputs(B, seed, ties)
     assert MO.state_change_accuracy(op, ol) == ref.state_change_accuracy(op, ol)
     assert MO.keyframe_accuracy(preds, labels, sc) == ref.keyframe_accuracy(preds, labels, sc)
