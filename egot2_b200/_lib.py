@@ -12,6 +12,8 @@ MAX_SEG = 8
 MAX_GROUPS = 4
 F32, BF16 = 0, 1
 LOSS_NONE, LOSS_CE, LOSS_BCE_SIGMOID, LOSS_CE_GROUPS = 0, 1, 2, 3
+LR_CONSTANT, LR_COSINE, LR_STEPS = 0, 1, 2
+LR_MAX_MILESTONES = 8
 
 # EGOT2_LIB: an alternative build of the same library (instrumented / experimental variants for tools/); never a fallback
 _LIB_PATH = os.environ.get("EGOT2_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libegot2.so")
@@ -102,7 +104,13 @@ class DpDesc(C.Structure):
     _fields_ = [("world", i32), ("rank", i32), ("numel", C.c_int64), ("slab", vp * 8), ("off_param", C.c_int64),
                 ("off_grad", C.c_int64), ("off_shadow", C.c_int64), ("off_flags", C.c_int64), ("exp_avg", vp), ("exp_avg_sq", vp),
                 ("lr", f32), ("beta1", f32), ("beta2", f32), ("eps", f32), ("weight_decay", f32), ("step", i32), ("step_dev", vp),
-                ("decoupled", i32), ("zero_grads_remote", i32)]
+                ("decoupled", i32), ("zero_grads_remote", i32), ("lr_dev", vp)]
+
+
+class LrSched(C.Structure):
+    _fields_ = [("kind", i32), ("n_milestones", i32), ("warmup_steps", C.c_int64), ("total_steps", C.c_int64),
+                ("base_lr", C.c_double), ("warmup_start_lr", C.c_double), ("end_lr", C.c_double),
+                ("milestones", C.c_int64 * LR_MAX_MILESTONES), ("factors", C.c_double * (LR_MAX_MILESTONES + 1))]
 
 
 class HeadGrads(C.Structure):
@@ -191,6 +199,8 @@ SIGNATURES = {
     "egot2_adam_step_fused": (C.c_int, [vp, vp, vp, vp, sz, f32, f32, f32, f32, f32, i32, f32, vp, i32, vp]),
     "egot2_adamw_step_fused": (C.c_int, [vp, vp, vp, vp, sz, f32, f32, f32, f32, f32, i32, f32, vp, i32, vp]),
     "egot2_adam_step_fused_dev": (C.c_int, [vp, vp, vp, vp, sz, f32, f32, f32, f32, f32, vp, f32, vp, i32, vp]),
+    "egot2_adam_step_fused_sched": (C.c_int, [vp, vp, vp, vp, sz, vp, f32, f32, f32, f32, vp, f32, vp, i32, i32, vp]),
+    "egot2_opt_advance": (C.c_int, [vp, vp, vp, vp]),
     "egot2_gemm": (C.c_int, [i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, i32, i32, vp]),
     "egot2_gemm_last_impl": (C.c_char_p, []),
     "egot2_layernorm_fwd": (C.c_int, [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp]),

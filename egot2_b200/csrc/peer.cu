@@ -41,6 +41,7 @@ struct DpArgs {
   float* m; float* v;                  // local Adam moments (full arena layout; only this rank's slice is used)
   float lr, b1, b2, eps, wd, bc1, bc2_sqrt;
   const int32_t* step_dev;             // optional: optimizer step count on the device (graph replays)
+  const float* lr_dev;                 // optional: learning rate on the device (egot2_opt_advance)
   int decoupled;
 };
 
@@ -84,6 +85,7 @@ __global__ void __launch_bounds__(256) dp_reduce_adam_kernel(const DpArgs a) {
     bc1 = 1.f - powf(a.b1, t);
     bc2_sqrt = sqrtf(1.f - powf(a.b2, t));
   }
+  const float lr = a.lr_dev ? *a.lr_dev : a.lr;
   const float inv_world = 1.f / (float)a.world;
   // slices in units of 4 floats (the arena is padded to a multiple of 64)
   const size_t n4 = (a.hi - a.lo) / 4, per = (n4 + a.world - 1) / a.world, base = a.lo / 4;
@@ -117,11 +119,11 @@ __global__ void __launch_bounds__(256) dp_reduce_adam_kernel(const DpArgs a) {
       for (int k = 0; k < 4; ++k) {              // the arithmetic of adam_kernel (rowops.cu), element for element
         float grad = gg[k];
         float wk = w[k];
-        if (a.decoupled) wk *= 1.f - a.lr * a.wd;
+        if (a.decoupled) wk *= 1.f - lr * a.wd;
         else if (a.wd != 0.f) grad += a.wd * wk;
         mm[k] = a.b1 * mm[k] + (1.f - a.b1) * grad;
         vv[k] = a.b2 * vv[k] + (1.f - a.b2) * grad * grad;
-        w[k] = wk - (a.lr / bc1) * mm[k] / (sqrtf(vv[k]) / bc2_sqrt + a.eps);
+        w[k] = wk - (lr / bc1) * mm[k] / (sqrtf(vv[k]) / bc2_sqrt + a.eps);
       }
       reinterpret_cast<float4*>(a.m)[q] = make_float4(mm[0], mm[1], mm[2], mm[3]);
       reinterpret_cast<float4*>(a.v)[q] = make_float4(vv[0], vv[1], vv[2], vv[3]);
@@ -225,6 +227,7 @@ static int dp_launch(const egot2_dp_desc* d, long long lo, long long hi, int cha
   a.bc1 = 1.f - powf(d->beta1, (float)d->step);
   a.bc2_sqrt = sqrtf(1.f - powf(d->beta2, (float)d->step));
   a.step_dev = d->step_dev;
+  a.lr_dev = d->lr_dev;
   a.decoupled = d->decoupled;
   // a few CTAs per rank: the message is latency-bound, and the spinning CTAs must never crowd out other work
   const size_t per4 = ((size_t)(hi - lo) / 4 + d->world - 1) / d->world;

@@ -384,13 +384,14 @@ template <bool DECOUPLED>
 __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, size_t n, float lr, float b1, float b2, float eps, float wd,
                             float bc1, float bc2_sqrt, float gscale, bf16* __restrict__ shadow, int zero_grad,
-                            const int32_t* __restrict__ step_dev) {
+                            const int32_t* __restrict__ step_dev, const float* __restrict__ lr_dev) {
   EGOT2_PDL_ENTER();
   if (step_dev) {            // step count kept on the device (whole-step CUDA graphs): bias corrections computed here
     const float t = (float)*step_dev;
     bc1 = 1.f - powf(b1, t);
     bc2_sqrt = sqrtf(1.f - powf(b2, t));
   }
+  if (lr_dev) lr = *lr_dev;  // learning-rate schedule evaluated on the device (egot2_opt_advance)
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     float grad = g[i] * gscale;
     float w = p[i];
@@ -405,6 +406,35 @@ __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float*
     if (shadow) shadow[i] = __float2bfloat16_rn(wn);     // the bf16 copy the next forward's GEMMs read
     if (zero_grad) g[i] = 0.f;                           // the next backward accumulates into a clean arena
   }
+}
+
+// lr_at of include/egot2.h, without the warm-up
+__device__ double lr_policy(const egot2_lr_sched& s, long long t) {
+  if (s.kind == EGOT2_LR_COSINE) {
+    if (t >= s.total_steps) return s.end_lr;
+    return s.end_lr + (s.base_lr - s.end_lr) * (1.0 + cos(M_PI * (double)t / (double)s.total_steps)) * 0.5;
+  }
+  if (s.kind == EGOT2_LR_STEPS) {
+    int i = 0;
+    while (i < s.n_milestones && i < 8 && s.milestones[i] <= t) ++i;
+    return s.base_lr * s.factors[i];
+  }
+  return s.base_lr;
+}
+__global__ void opt_advance_kernel(int32_t* __restrict__ step, const egot2_lr_sched* __restrict__ sched, float* __restrict__ lr) {
+  EGOT2_PDL_ENTER();
+  const egot2_lr_sched s = *sched;
+  const int32_t t = *step + 1;
+  const long long k = t - 1;           // lr of optimizer step t = lr_at(t - 1)
+  double v;
+  if (k < s.warmup_steps) {
+    const double w0 = s.warmup_start_lr;
+    v = w0 + (lr_policy(s, s.warmup_steps) - w0) * (double)k / (double)s.warmup_steps;
+  } else {
+    v = lr_policy(s, k);
+  }
+  *step = t;
+  *lr = (float)v;
 }
 
 struct SegList { int n; int tokens[EGOT2_MAX_SEG]; int task[EGOT2_MAX_SEG]; };
@@ -991,7 +1021,8 @@ extern "C" int egot2_cast_bf16_to_f32(const void* src, float* dst, size_t n, voi
 
 static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr, float beta1,
                        float beta2, float eps, float weight_decay, int32_t step, float grad_scale, void* shadow,
-                       int zero_grad, void* stream, const int32_t* step_dev = nullptr, bool decoupled = false) {
+                       int zero_grad, void* stream, const int32_t* step_dev = nullptr, bool decoupled = false,
+                       const float* lr_dev = nullptr) {
   EGOT2_CHECK(step >= 1 || step_dev, "adam: step must be >= 1");
   if (n == 0) return 0;
   const float bc1 = 1.f - powf(beta1, (float)step);
@@ -999,10 +1030,10 @@ static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg
   ProfScope prof((cudaStream_t)stream, "adam n%zu", n);
   if (decoupled)
     launch(adam_kernel<true>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev);
+           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev);
   else
     launch(adam_kernel<false>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev);
+           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev);
   EGOT2_LAUNCH_CHECK();
   return 0;
 }
@@ -1034,6 +1065,22 @@ extern "C" int egot2_adam_step_fused_dev(float* param, float* grad, float* exp_a
   EGOT2_CHECK(step_dev != nullptr, "adam: step_dev is null");
   return adam_launch(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, 1, grad_scale, shadow_bf16,
                      zero_grad, stream, step_dev);
+}
+
+extern "C" int egot2_adam_step_fused_sched(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n,
+                                           const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                           const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                                           int32_t decoupled, void* stream) {
+  EGOT2_CHECK(step_dev != nullptr && lr_dev != nullptr, "adam: step_dev / lr_dev is null");
+  return adam_launch(param, grad, exp_avg, exp_avg_sq, n, 0.f, beta1, beta2, eps, weight_decay, 1, grad_scale, shadow_bf16,
+                     zero_grad, stream, step_dev, decoupled != 0, lr_dev);
+}
+
+extern "C" int egot2_opt_advance(int32_t* step_dev, const egot2_lr_sched* sched, float* lr_dev, void* stream) {
+  EGOT2_CHECK(step_dev && sched && lr_dev, "opt_advance: step_dev / sched / lr_dev is null");
+  launch(opt_advance_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, step_dev, sched, lr_dev);
+  EGOT2_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" int egot2_hhi_tok_table_fwd(const float* task_embed, const float* pe, int32_t pe_len, int32_t n_seg,

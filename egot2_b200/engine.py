@@ -138,14 +138,16 @@ class ParamArena:
         ow, ob = self.offsets[w0], self.offsets[b0]
         return base[ow:ow + rows * H].view(rows, H), base[ob:ob + rows]
 
-    def load_state_dict(self, sd: Dict[str, torch.Tensor]):
+    def load_state_dict(self, sd: Dict[str, torch.Tensor], base: Optional[torch.Tensor] = None):
+        """base: another buffer of the arena's layout (e.g. Adam moments) to fill instead of the parameters."""
         with torch.no_grad():
             for name in self.shapes:
-                self.view(name).copy_(sd[name].to(device=self.device, dtype=torch.float32))
-        self.shadow_fresh = False
+                self.view(name, base).copy_(sd[name].to(device=self.device, dtype=torch.float32))
+        if base is None:
+            self.shadow_fresh = False
 
-    def state_dict(self) -> Dict[str, torch.Tensor]:
-        return {name: self.view(name).clone() for name in self.shapes}
+    def state_dict(self, base: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        return {name: self.view(name, base).clone() for name in self.shapes}
 
     @_on_device
     def refresh_shadow(self):
@@ -788,21 +790,32 @@ class TranslatorEngine:
     @_on_device
     def adam_step(self, state: Dict[str, torch.Tensor], step: int, lr: float = 5e-4, betas=(0.9, 0.999),
                   eps: float = 1e-8, weight_decay: float = 0.0, grad_scale: float = 1.0, fused: bool = False,
-                  step_dev: Optional[torch.Tensor] = None, decoupled: bool = False):
+                  step_dev: Optional[torch.Tensor] = None, decoupled: bool = False, lr_dev: Optional[torch.Tensor] = None):
         """torch.optim.Adam over the whole arena in one launch (HHI/tasks/ttm/video_task.py:64-66: lr 5e-4).
         fused: the same launch also writes the bf16 shadow of the updated parameters (bf16 engines) and clears the
         gradient arena, so the next step needs neither the cast launch nor a fill (callers then pass
-        zero_grad=False to backward())."""
+        zero_grad=False to backward()).
+        step_dev / lr_dev: the step count (int32) and the learning rate (float32) are read from device memory when the
+        kernel executes (graph replays, device-evaluated schedules: optim.py); lr_dev needs step_dev."""
         if "m" not in state:
             state["m"] = torch.zeros_like(self.arena.param)
             state["v"] = torch.zeros_like(self.arena.param)
+        if lr_dev is not None and step_dev is None:
+            raise L.Egot2Error("adam_step: lr_dev needs step_dev (egot2_opt_advance keeps both on the device)")
         if fused:
             shadow = None
             if self.dtype == "bf16":
                 if self.arena.shadow is None:
                     self.arena.refresh_shadow()
                 shadow = self.arena.shadow.data_ptr()
-            if step_dev is not None:        # step count read on the device (graph-resident update)
+            if step_dev is not None and (lr_dev is not None or decoupled):
+                if lr_dev is None:          # AdamW with a device step count: the fixed lr goes to the device as well
+                    lr_dev = torch.full((1,), float(lr), device=self.device, dtype=torch.float32)
+                L.call("egot2_adam_step_fused_sched", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
+                       state["m"].data_ptr(), state["v"].data_ptr(), self.arena.numel, lr_dev.data_ptr(), betas[0],
+                       betas[1], eps, weight_decay, step_dev.data_ptr(), float(grad_scale), shadow, 1,
+                       1 if decoupled else 0, _stream())
+            elif step_dev is not None:      # step count read on the device (graph-resident update)
                 L.call("egot2_adam_step_fused_dev", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
                        state["m"].data_ptr(), state["v"].data_ptr(), self.arena.numel, lr, betas[0], betas[1], eps,
                        weight_decay, step_dev.data_ptr(), float(grad_scale), shadow, 1, _stream())

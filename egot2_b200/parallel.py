@@ -168,9 +168,10 @@ class PeerExchange:
         self.desc.off_param, self.desc.off_grad, self.desc.off_shadow, self.desc.off_flags = off_param, off_grad, off_shadow, off_flags
 
     def step(self, state, step: int, hp, stream: int, step_dev: Optional[torch.Tensor] = None, decoupled: bool = False,
-             lo: int = 0, hi: Optional[int] = None, channel: int = 0):
+             lo: int = 0, hi: Optional[int] = None, channel: int = 0, lr_dev: Optional[torch.Tensor] = None):
         """The exchange + optimizer step of this rank for arena elements [lo, hi) (default: everything) on flag `channel`;
-        afterwards that part of the gradient arena is cleared (stream order)."""
+        afterwards that part of the gradient arena is cleared (stream order).  lr_dev: the learning rate is read from this
+        device float when the kernel executes (optim.py), instead of hp["lr"]."""
         import ctypes as C
         from . import _lib as L
         arena = self.engine.arena
@@ -182,6 +183,7 @@ class PeerExchange:
         d.lr, (d.beta1, d.beta2), d.eps, d.weight_decay = hp["lr"], hp["betas"], hp["eps"], hp["weight_decay"]
         d.step = int(step)
         d.step_dev = step_dev.data_ptr() if step_dev is not None else None
+        d.lr_dev = lr_dev.data_ptr() if lr_dev is not None else None
         d.decoupled = 1 if decoupled else 0
         hi = arena.numel if hi is None else hi
         # small exchanges: the slice owners clear the gradients in the same kernel; large ones: one local clear afterwards

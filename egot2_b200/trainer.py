@@ -12,12 +12,14 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Sequence
 
+import ctypes as C
 import os
 
 import torch
 
 from . import _lib as L
 from .engine import Activations, TranslatorEngine
+from .optim import LRSchedule
 from .parallel import allreduce_gradients
 from .specs import TranslatorSpec
 
@@ -56,7 +58,97 @@ def _make_peer_exchange(engine, process_group, world):
     return peer if int(flag.item()) == 1 else None
 
 
-class _PromptStepGraphs:
+class _OptimizerState:
+    """Learning-rate schedule and resumable optimizer state of the fused trainers.
+
+    With `lr_schedule` (optim.LRSchedule) the trainer owns three device buffers: the egot2_lr_sched descriptor, the lr of
+    the last step and the optimizer step count.  Every step, on every path, is egot2_opt_advance (step count + 1, lr of
+    that step) followed by an optimizer launch that reads both from the device, so a replayed CUDA graph follows the
+    schedule and `set_lr_schedule` takes effect without a new capture.  Without a schedule nothing here adds a launch."""
+
+    def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float):
+        if lr_schedule is not None and lr != default_lr:
+            raise ValueError("pass either lr or lr_schedule, not both")
+        self.lr_schedule = None
+        self._epoch = 0                    # dropout epoch of the next step: the trainer advances it once per step from 0
+        if not hasattr(self, "_step_dev"):
+            self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
+            self._step_dev_val = 0
+        if lr_schedule is not None:
+            self._sched_dev = torch.zeros(C.sizeof(L.LrSched), device=self.device, dtype=torch.uint8)
+            self._lr_dev = torch.zeros(1, device=self.device, dtype=torch.float32)
+            self.lr_schedule = lr_schedule
+            self.set_lr_schedule(lr_schedule)
+
+    def set_lr_schedule(self, schedule: LRSchedule):
+        """Rewrite the device descriptor (in stream order): the next step follows `schedule` at its current step count, in
+        graph mode without a new capture.  To drive the lr from host code, call set_lr_schedule(LRSchedule.constant(x))
+        before each step."""
+        if self.lr_schedule is None:
+            raise ValueError("this trainer was built without lr_schedule; its optimizer launches take hp['lr']")
+        host = torch.frombuffer(bytearray(bytes(schedule.pack())), dtype=torch.uint8)
+        # pageable source: the copy is staged before copy_ returns, so `host` may go away at once
+        self._sched_dev.copy_(host, non_blocking=True)
+        self.lr_schedule = schedule
+
+    @property
+    def last_lr(self) -> torch.Tensor:
+        """The lr the last step used, as a 0-dim device tensor (with a schedule a view of the device lr: no sync)."""
+        if self.lr_schedule is None:
+            return torch.tensor(float(self.hp["lr"]), device=self.device)
+        return self._lr_dev[0]
+
+    def _opt_advance(self, stream: int):
+        with _dev_guard(self.device):
+            L.call("egot2_opt_advance", self._step_dev.data_ptr(), self._sched_dev.data_ptr(), self._lr_dev.data_ptr(),
+                   stream)
+
+    def _advance_eager(self) -> dict:
+        """Before an eager optimizer launch: with a schedule, advance the device step count and lr on the current stream
+        and return the launch's step_dev / lr_dev arguments; without one, nothing ({})."""
+        if self.lr_schedule is None:
+            return {}
+        if self._step_dev_val != self.step_count - 1:
+            self._step_dev.fill_(self.step_count - 1)
+        self._opt_advance(_cur_stream(self.device))
+        self._step_dev_val = self.step_count
+        return dict(step_dev=self._step_dev, lr_dev=self._lr_dev)
+
+    def optimizer_state_dict(self) -> dict:
+        """What a run needs beyond the parameters (state_dict) to resume as if uninterrupted: the Adam moments keyed by
+        parameter name, the step count, the schedule and the dropout epoch.  Under the peer-memory exchange every rank
+        holds the moments of its own arena slice only: save and load per rank."""
+        arena = self.engine.arena
+        zeros = None if "m" in self.opt_state else torch.zeros_like(arena.param)
+        return {"step": self.step_count,
+                "exp_avg": arena.state_dict(self.opt_state.get("m", zeros)),
+                "exp_avg_sq": arena.state_dict(self.opt_state.get("v", zeros)),
+                "lr_schedule": None if self.lr_schedule is None else self.lr_schedule.to_dict(),
+                "dropout_epoch": self._epoch}
+
+    def load_optimizer_state_dict(self, sd: dict):
+        if (sd["lr_schedule"] is None) != (self.lr_schedule is None):
+            raise ValueError("optimizer state saved " + ("without" if sd["lr_schedule"] is None else "with") +
+                             " an lr_schedule: build the trainer the same way")
+        arena = self.engine.arena
+        for k, key in (("m", "exp_avg"), ("v", "exp_avg_sq")):
+            if k in self.opt_state:        # in place: captured graphs hold these buffers
+                self.opt_state[k].zero_()
+            else:
+                self.opt_state[k] = torch.zeros_like(arena.param)
+            arena.load_state_dict(sd[key], base=self.opt_state[k])
+        self.step_count = int(sd["step"])
+        self._step_dev.fill_(self.step_count)
+        self._step_dev_val = self.step_count
+        if self.lr_schedule is not None:
+            self.set_lr_schedule(LRSchedule.from_dict(sd["lr_schedule"]))
+        self._epoch = int(sd["dropout_epoch"])
+        if self.dropout_epoch:
+            with _dev_guard(self.device):
+                L.call("egot2_dropout_epoch_set", self._epoch, _cur_stream(self.device))
+
+
+class _PromptStepGraphs(_OptimizerState):
     """Optional CUDA-graph replay of an EgoT2-g step's forward/backward launch sequence (several hundred small eager
     launches per step otherwise).  On by default since it ran green on hardware (round 2); EGOT2_G_GRAPH=0 keeps eager
     launches.  One graph per `graph_key` (= one fixed set of input
@@ -107,17 +199,20 @@ class _PromptStepGraphs:
             arena.refresh_shadow()
         replay()
         if getattr(self, "peer", None) is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=decoupled)
+            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=decoupled,
+                           **self._advance_eager())
         else:
             scale = 1.0
             if self.world > 1:
                 scale = allreduce_gradients(arena.grad, self.pg)
             self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                                  self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=decoupled)
+                                  self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=decoupled,
+                                  **self._advance_eager())
         self._grad_clean = True
         if self.dropout_epoch:
             with _dev_guard(self.device):
                 L.call("egot2_dropout_epoch_advance", _cur_stream(self.device))
+            self._epoch += 1
         return total
 
 
@@ -131,7 +226,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
                  labels = the three (rows_i, 3) target-token tensors concatenated along rows."""
 
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
-                 ratios=(1.0, 1.0, 1.0), process_group=None):
+                 ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -161,6 +256,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
+        self._init_optimizer_state(lr_schedule, lr, 5e-4)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -211,15 +307,16 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
             self.engine.arena.grad.zero_()
         total = self._fwd_bwd_all(feats, labels, self.step_count * 4)         # one arena, accumulated over the three
         if self.peer is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device))
+            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), **self._advance_eager())
             self._grad_clean = True
             return total
         scale = 1.0
         if self.world > 1:
             scale = allreduce_gradients(self.engine.arena.grad, self.pg)
+        sched = self._advance_eager()      # a schedule needs the fused launch (the one that reads the device lr)
         self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                              self.hp["weight_decay"], grad_scale=scale)
-        self._grad_clean = False           # the plain Adam launch leaves the gradients in place
+                              self.hp["weight_decay"], grad_scale=scale, fused=bool(sched), **sched)
+        self._grad_clean = bool(sched)     # the plain Adam launch leaves the gradients in place
         return total
 
     train_stream_host = None     # bound below to TranslatorTrainer's implementation (same double-buffered host path)
@@ -235,7 +332,8 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
     Step inputs: feats = 3 x [pnr, oscc, slow, fast] (12 tensors), labels = the three target tensors concatenated."""
 
     def __init__(self, hidden=512, heads=8, layers=3, dropout=0.1, vocab=600, device="cuda:0", dtype: str = "bf16",
-                 lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None):
+                 lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
+                 lr_schedule: Optional[LRSchedule] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -267,6 +365,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
+        self._init_optimizer_state(lr_schedule, lr, 1e-4)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -321,7 +420,8 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
             l = act.t["loss"][0] * ratio
             total = l if total is None else total + l
         if self.peer is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=True)
+            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=True,
+                           **self._advance_eager())
             self._grad_clean = True
             return total
         scale = 1.0
@@ -329,7 +429,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
             scale = allreduce_gradients(eng.arena.grad, self.pg)
         # AdamW (decoupled decay) + bf16 shadow + gradient clear in one launch
         eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=True)
+                      self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=True, **self._advance_eager())
         self._grad_clean = True
         return total
 
@@ -345,10 +445,10 @@ def default_loss(spec: TranslatorSpec):
     raise ValueError(f"{spec.family}: the loss lives outside the translator (use the nn.Module API)")
 
 
-class TranslatorTrainer:
+class TranslatorTrainer(_OptimizerState):
     def __init__(self, spec: TranslatorSpec, device, dtype: str = "bf16", lr: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
-                 sinusoid: Optional[torch.Tensor] = None):
+                 sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -401,6 +501,7 @@ class TranslatorTrainer:
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
+        self._init_optimizer_state(lr_schedule, lr, 5e-4)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}
@@ -430,6 +531,8 @@ class TranslatorTrainer:
         dropout epoch (advanced once per step, folded into every key at execution time) makes each replay draw fresh
         masks all the same."""
         self.step_count += 1
+        if self.dropout_epoch:
+            self._epoch += 1               # every path below advances the device epoch once
         if graph_key is not None and self.use_graphs:
             entry = self._graphs.get(graph_key)
             if entry is None:
@@ -471,7 +574,7 @@ class TranslatorTrainer:
         dist.all_reduce(eng.arena.grad[:nb], group=self.pg)
         work.wait()
         eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=1.0 / self.world, fused=True)
+                      self.hp["weight_decay"], grad_scale=1.0 / self.world, fused=True, **self._advance_eager())
         self._grad_clean = True
         self._advance_epoch()
         return act.t["loss"][0]
@@ -520,7 +623,10 @@ class TranslatorTrainer:
             if self.graph_update:                         # side branch: advance the device-resident step count
                 self._bump_stream.wait_stream(cur)
                 with torch.cuda.stream(self._bump_stream):
-                    self._step_dev.add_(1)
+                    if self.lr_schedule is not None:      # ... and the lr of that step
+                        self._opt_advance(self._bump_stream.cuda_stream)
+                    else:
+                        self._step_dev.add_(1)
             split = self.graph_update and self.peer is not None and self.engine.spec.head != "decoder" \
                 and os.environ.get("EGOT2_DP_SPLIT", "0") == "1"
             if split:
@@ -533,13 +639,13 @@ class TranslatorTrainer:
                 self._peer_stream.wait_stream(cur)
                 with torch.cuda.stream(self._peer_stream):
                     self.peer.step(self.opt_state, self.step_count, self.hp, self._peer_stream.cuda_stream,
-                                   step_dev=self._step_dev, lo=nb, hi=n, channel=0)
+                                   step_dev=self._step_dev, lo=nb, hi=n, channel=0, lr_dev=self._graph_lr_dev())
                 self.engine.backward(act, zero_grad=False, stage="embed")
                 self._bump_stream.wait_stream(cur)
                 with torch.cuda.stream(self._bump_stream):
                     self._advance_epoch()
                 self.peer.step(self.opt_state, self.step_count, self.hp, cur.cuda_stream, step_dev=self._step_dev,
-                               lo=0, hi=nb, channel=1)
+                               lo=0, hi=nb, channel=1, lr_dev=self._graph_lr_dev())
                 cur.wait_stream(self._peer_stream)
                 cur.wait_stream(self._bump_stream)
                 self._grad_clean = True
@@ -569,18 +675,27 @@ class TranslatorTrainer:
             with _dev_guard(self.device):
                 L.call("egot2_dropout_epoch_advance", torch.cuda.current_stream(self.device).cuda_stream)      # current = the stream in effect
 
+    def _graph_lr_dev(self) -> Optional[torch.Tensor]:
+        """lr_dev of an optimizer launch inside the whole-step graph (advanced on its side branch), None without a schedule."""
+        return None if self.lr_schedule is None else self._lr_dev
+
     def _reduce_and_update(self, step_dev: Optional[torch.Tensor] = None):
+        """step_dev: the launch sits in the whole-step graph, whose side branch advances the step count (and lr)."""
         eng = self.engine
+        if step_dev is None:
+            opt = self._advance_eager()
+        else:
+            opt = dict(step_dev=step_dev, lr_dev=self._graph_lr_dev())
         if self.peer is not None:                         # one kernel: reduce-scatter + Adam + all-gather over peer memory
             self.peer.step(self.opt_state, self.step_count, self.hp, torch.cuda.current_stream(self.device).cuda_stream,
-                           step_dev=step_dev)
+                           **opt)
             self._grad_clean = True
             return
         scale = 1.0
         if self.world > 1:
             scale = allreduce_gradients(eng.arena.grad, self.pg)            # ONE flat NCCL all-reduce (NVLink)
         eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=scale, fused=True, step_dev=step_dev)
+                      self.hp["weight_decay"], grad_scale=scale, fused=True, **opt)
         self._grad_clean = True
 
     # ------------------------------------------------------------------ host-buffer (end-to-end) step

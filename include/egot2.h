@@ -32,6 +32,10 @@
  *                                HOI/models/pnr/simple_vit.py:55-107, HOI/models/pnr/video_model_transfer_3task.py:128-164
  *   egot2_adam_step              torch.optim.Adam over the flat translator parameter arena
  *                                HHI/tasks/ttm/video_task.py:64-66
+ *   egot2_opt_advance            the optimizer step count and the learning rate of that step, on the device: the
+ *                                warm-up + cosine / step-wise schedules of the HOI recipes (SURVEY.md §3.5,
+ *                                HOI/optimizers/lta/lr_scheduler.py:21-26,67-91), read by egot2_adam_step_fused_sched
+ *                                and by egot2_dp_reduce_adam (egot2_dp_desc.lr_dev) when they execute
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -401,6 +405,32 @@ int egot2_adamw_step_fused(float* param, float* grad, float* exp_avg, float* exp
                            float beta1, float beta2, float eps, float weight_decay, int32_t step, float grad_scale,
                            void* shadow_bf16, int32_t zero_grad, void* stream);
 
+/* Learning-rate schedule, evaluated on the device.  lr_at(s) for optimizer step s = 0, 1, ... (fp64, rounded once to float):
+ *   CONSTANT  base_lr
+ *   COSINE    end_lr + (base_lr - end_lr) * (1 + cos(pi * s / total_steps)) / 2, and end_lr for s >= total_steps
+ *   STEPS     base_lr * factors[i], i = the number of milestones <= s (SlowFast's steps-with-relative-lrs; MultiStepLR
+ *             when factors[i] = gamma^i); milestones increasing, n_milestones <= 8, factors[0..n_milestones] used
+ * and, for every kind, a linear warm-up over s < warmup_steps:
+ *             warmup_start_lr + (lr_at(warmup_steps) - warmup_start_lr) * s / warmup_steps.
+ * The lr of optimizer step t (1-based) is lr_at(t - 1): torch.optim.lr_scheduler.LambdaLR stepped after every
+ * optimizer.step(). */
+enum { EGOT2_LR_CONSTANT = 0, EGOT2_LR_COSINE = 1, EGOT2_LR_STEPS = 2 };
+typedef struct {
+  int32_t kind, n_milestones;           /* EGOT2_LR_*; STEPS: <= 8 */
+  int64_t warmup_steps, total_steps;    /* in optimizer steps; total_steps > 0 for COSINE */
+  double base_lr, warmup_start_lr, end_lr;
+  int64_t milestones[8];
+  double factors[9];
+} egot2_lr_sched;
+/* One thread: t = ++*step_dev; *lr_dev = (float) lr_at(*sched, t - 1).  All three are DEVICE pointers, read when the kernel
+ * executes, so a CUDA graph that contains the launch follows a schedule rewritten between replays. */
+int egot2_opt_advance(int32_t* step_dev, const egot2_lr_sched* sched, float* lr_dev, void* stream);
+/* egot2_adam_step_fused_dev with the learning rate read from DEVICE memory (*lr_dev, e.g. written by egot2_opt_advance) at
+ * execution time; decoupled = 1 runs AdamW (param *= 1 - lr*weight_decay with the same device lr). */
+int egot2_adam_step_fused_sched(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, const float* lr_dev,
+                                float beta1, float beta2, float eps, float weight_decay, const int32_t* step_dev,
+                                float grad_scale, void* shadow_bf16, int32_t zero_grad, int32_t decoupled, void* stream);
+
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
  * translator gradients after backward, then the optimizer on every rank.  Here that is ONE kernel (csrc/peer.cu): gradient
@@ -426,6 +456,7 @@ typedef struct {
   int32_t decoupled;                  /* 1: AdamW */
   int32_t zero_grads_remote;          /* 1: the owner of a slice clears that slice of every rank's gradient arena after reading
                                        * it (small arenas: no separate clear launch); 0: the caller clears its arena afterwards */
+  const float* lr_dev;                /* optional: the learning rate lives on the device (egot2_opt_advance); NULL: `lr` */
 } egot2_dp_desc;
 int egot2_peer_alloc(size_t bytes, void** ptr);
 int egot2_peer_free(void* ptr);
