@@ -187,4 +187,37 @@ int loss_fwd(const egot2_head_desc& d, int rows, const float* logits, const int6
 int loss_bwd(const egot2_head_desc& d, int rows, const float* logits, const int64_t* labels, const float* class_weight,
              const float* loss2, float dloss_scale, float* dlogits, cudaStream_t st);
 
+// ---- gradient guard (egot2_grad_guard): shared by egot2_grad_norm (rowops.cu) and the guarded peer exchange (peer.cu)
+// Sum of v over the CTA in a fixed order (shuffle tree per warp, then the warp sums in warp order); the result is valid in
+// thread 0.  `sh` holds blockDim.x / 32 doubles; every thread of the CTA must call it.
+__device__ __forceinline__ double block_sum_f64(double v, double* sh) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  const int warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  __syncthreads();                     // `sh` may still be read by a previous call
+  if ((threadIdx.x & 31) == 0) sh[warp] = v;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0)
+    for (int w = 0; w < nw; ++w) s += sh[w];
+  return s;
+}
+// total_norm = sqrt(sumsq) * |scale|; a finite norm gives the clip coefficient, a non-finite one skips the step and
+// takes back the step-count increment of this step (so the count, the bias corrections and the lr schedule count applied
+// steps only).  One thread.
+__device__ __forceinline__ void grad_guard_finalize(double sumsq, float scale, egot2_grad_guard* guard, int32_t* step_dev) {
+  const double tot = sqrt(sumsq) * fabs((double)scale);
+  const float tn = (float)tot;
+  guard->total_norm = tn;
+  if (isfinite(tot)) {
+    guard->coef = fminf(1.f, guard->max_norm / (tn + 1e-6f));      // clip_grad_norm_: clamp(max_norm / (norm + 1e-6), max=1)
+    guard->skip = 0;
+  } else {
+    guard->coef = 0.f;
+    guard->skip = 1;
+    guard->skipped += 1;
+    if (step_dev) *step_dev -= 1;
+  }
+}
+
 }  // namespace egot2

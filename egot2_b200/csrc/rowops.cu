@@ -384,8 +384,17 @@ template <bool DECOUPLED>
 __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, size_t n, float lr, float b1, float b2, float eps, float wd,
                             float bc1, float bc2_sqrt, float gscale, bf16* __restrict__ shadow, int zero_grad,
-                            const int32_t* __restrict__ step_dev, const float* __restrict__ lr_dev) {
+                            const int32_t* __restrict__ step_dev, const float* __restrict__ lr_dev,
+                            const egot2_grad_guard* __restrict__ guard) {
   EGOT2_PDL_ENTER();
+  if (guard) {               // egot2_grad_norm ran before: clip, or skip the update and only clear the gradient
+    if (guard->skip) {
+      if (zero_grad)
+        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) g[i] = 0.f;
+      return;
+    }
+    gscale *= guard->coef;
+  }
   if (step_dev) {            // step count kept on the device (whole-step CUDA graphs): bias corrections computed here
     const float t = (float)*step_dev;
     bc1 = 1.f - powf(b1, t);
@@ -435,6 +444,53 @@ __global__ void opt_advance_kernel(int32_t* __restrict__ step, const egot2_lr_sc
   }
   *step = t;
   *lr = (float)v;
+}
+
+// egot2_grad_norm: a fixed grid (not sm_count-dependent, so every GPU adds in the same order), fp64 squares per thread in
+// index order, a fixed-order CTA sum, and the last CTA to finish adds the per-CTA sums in CTA order.
+constexpr int kNormCtas = 512, kNormThreads = 256;
+__global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const float* __restrict__ g, size_t n, float scale,
+                                                                 egot2_grad_guard* __restrict__ guard, int32_t* step_dev,
+                                                                 double* part, unsigned int* ctr) {
+  EGOT2_PDL_ENTER();
+  __shared__ double sh[kNormThreads / 32];
+  __shared__ unsigned int s_last;
+  const size_t tid = blockIdx.x * (size_t)kNormThreads + threadIdx.x, stride = (size_t)kNormCtas * kNormThreads;
+  double s = 0.0;
+  size_t tail = 0;
+  if ((reinterpret_cast<uintptr_t>(g) & 15) == 0) {
+    const float4* g4 = reinterpret_cast<const float4*>(g);
+    const size_t n4 = n / 4;
+    constexpr int U = 4;                 // independent loads in flight per thread
+    for (size_t q = tid; q < n4; q += stride * U) {
+      float4 x[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) x[u] = q + u * stride < n4 ? g4[q + u * stride] : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        s += (double)x[u].x * x[u].x; s += (double)x[u].y * x[u].y;
+        s += (double)x[u].z * x[u].z; s += (double)x[u].w * x[u].w;
+      }
+    }
+    tail = n4 * 4;
+  }
+  for (size_t i = tail + tid; i < n; i += stride) s += (double)g[i] * g[i];
+  s = block_sum_f64(s, sh);
+  if (threadIdx.x == 0) {
+    part[blockIdx.x] = s;
+    __threadfence();
+    s_last = atomicAdd(ctr, 1u) == kNormCtas - 1 ? 1u : 0u;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();                       // every CTA's fenced partial is visible to the last one
+  double t = 0.0;
+  for (int c = threadIdx.x; c < kNormCtas; c += kNormThreads) t += reinterpret_cast<volatile double*>(part)[c];
+  t = block_sum_f64(t, sh);
+  if (threadIdx.x == 0) {
+    grad_guard_finalize(t, scale, guard, step_dev);
+    *ctr = 0;                            // ready for the next launch (graph replays)
+  }
 }
 
 struct SegList { int n; int tokens[EGOT2_MAX_SEG]; int task[EGOT2_MAX_SEG]; };
@@ -1022,7 +1078,7 @@ extern "C" int egot2_cast_bf16_to_f32(const void* src, float* dst, size_t n, voi
 static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr, float beta1,
                        float beta2, float eps, float weight_decay, int32_t step, float grad_scale, void* shadow,
                        int zero_grad, void* stream, const int32_t* step_dev = nullptr, bool decoupled = false,
-                       const float* lr_dev = nullptr) {
+                       const float* lr_dev = nullptr, const egot2_grad_guard* guard = nullptr) {
   EGOT2_CHECK(step >= 1 || step_dev, "adam: step must be >= 1");
   if (n == 0) return 0;
   const float bc1 = 1.f - powf(beta1, (float)step);
@@ -1030,10 +1086,10 @@ static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg
   ProfScope prof((cudaStream_t)stream, "adam n%zu", n);
   if (decoupled)
     launch(adam_kernel<true>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev);
+           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev, guard);
   else
     launch(adam_kernel<false>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev);
+           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev, guard);
   EGOT2_LAUNCH_CHECK();
   return 0;
 }
@@ -1074,6 +1130,31 @@ extern "C" int egot2_adam_step_fused_sched(float* param, float* grad, float* exp
   EGOT2_CHECK(step_dev != nullptr && lr_dev != nullptr, "adam: step_dev / lr_dev is null");
   return adam_launch(param, grad, exp_avg, exp_avg_sq, n, 0.f, beta1, beta2, eps, weight_decay, 1, grad_scale, shadow_bf16,
                      zero_grad, stream, step_dev, decoupled != 0, lr_dev);
+}
+
+extern "C" int egot2_adam_step_fused_guard(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
+                                           const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                           const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                                           int32_t decoupled, const egot2_grad_guard* guard, void* stream) {
+  EGOT2_CHECK(step_dev != nullptr && guard != nullptr, "adam: step_dev / guard is null");
+  return adam_launch(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, 1, grad_scale, shadow_bf16,
+                     zero_grad, stream, step_dev, decoupled != 0, lr_dev, guard);
+}
+
+extern "C" size_t egot2_grad_norm_workspace_bytes(void) { return kNormCtas * sizeof(double) + 16; }
+
+extern "C" int egot2_grad_norm(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev,
+                               void* workspace, size_t ws_bytes, void* stream) {
+  EGOT2_CHECK(guard && workspace && (grad || n == 0), "grad_norm: grad / guard / workspace is null");
+  EGOT2_CHECK(ws_bytes >= egot2_grad_norm_workspace_bytes() && reinterpret_cast<uintptr_t>(workspace) % 8 == 0,
+              "grad_norm: workspace of %zu bytes (8-byte aligned) needed, got %zu", egot2_grad_norm_workspace_bytes(), ws_bytes);
+  double* part = (double*)workspace;
+  unsigned int* ctr = (unsigned int*)(part + kNormCtas);
+  ProfScope prof((cudaStream_t)stream, "grad_norm n%zu", n);
+  launch(grad_norm_kernel, dim3(kNormCtas), dim3(kNormThreads), 0, (cudaStream_t)stream, grad, n, grad_scale, guard, step_dev,
+         part, ctr);
+  EGOT2_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" int egot2_opt_advance(int32_t* step_dev, const egot2_lr_sched* sched, float* lr_dev, void* stream) {

@@ -790,25 +790,39 @@ class TranslatorEngine:
     @_on_device
     def adam_step(self, state: Dict[str, torch.Tensor], step: int, lr: float = 5e-4, betas=(0.9, 0.999),
                   eps: float = 1e-8, weight_decay: float = 0.0, grad_scale: float = 1.0, fused: bool = False,
-                  step_dev: Optional[torch.Tensor] = None, decoupled: bool = False, lr_dev: Optional[torch.Tensor] = None):
+                  step_dev: Optional[torch.Tensor] = None, decoupled: bool = False, lr_dev: Optional[torch.Tensor] = None,
+                  guard: Optional[torch.Tensor] = None):
         """torch.optim.Adam over the whole arena in one launch (HHI/tasks/ttm/video_task.py:64-66: lr 5e-4).
         fused: the same launch also writes the bf16 shadow of the updated parameters (bf16 engines) and clears the
         gradient arena, so the next step needs neither the cast launch nor a fill (callers then pass
         zero_grad=False to backward()).
         step_dev / lr_dev: the step count (int32) and the learning rate (float32) are read from device memory when the
-        kernel executes (graph replays, device-evaluated schedules: optim.py); lr_dev needs step_dev."""
+        kernel executes (graph replays, device-evaluated schedules: optim.py); lr_dev needs step_dev.
+        guard: a device egot2_grad_guard (_lib.GradGuard bytes; fused, needs step_dev): egot2_grad_norm of grad_scale * the
+        gradient arena first, then the update clipped by that norm, or skipped (gradient cleared, step count taken back)
+        when it is not finite."""
         if "m" not in state:
             state["m"] = torch.zeros_like(self.arena.param)
             state["v"] = torch.zeros_like(self.arena.param)
         if lr_dev is not None and step_dev is None:
             raise L.Egot2Error("adam_step: lr_dev needs step_dev (egot2_opt_advance keeps both on the device)")
+        if guard is not None and (step_dev is None or not fused):
+            raise L.Egot2Error("adam_step: a gradient guard needs the fused launch and step_dev (a skip takes the step back)")
         if fused:
             shadow = None
             if self.dtype == "bf16":
                 if self.arena.shadow is None:
                     self.arena.refresh_shadow()
                 shadow = self.arena.shadow.data_ptr()
-            if step_dev is not None and (lr_dev is not None or decoupled):
+            if guard is not None:
+                ws = self.grad_norm_workspace()
+                L.call("egot2_grad_norm", self.arena.grad.data_ptr(), self.arena.numel, float(grad_scale), guard.data_ptr(),
+                       step_dev.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
+                L.call("egot2_adam_step_fused_guard", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
+                       state["m"].data_ptr(), state["v"].data_ptr(), self.arena.numel, float(lr),
+                       None if lr_dev is None else lr_dev.data_ptr(), betas[0], betas[1], eps, weight_decay,
+                       step_dev.data_ptr(), float(grad_scale), shadow, 1, 1 if decoupled else 0, guard.data_ptr(), _stream())
+            elif step_dev is not None and (lr_dev is not None or decoupled):
                 if lr_dev is None:          # AdamW with a device step count: the fixed lr goes to the device as well
                     lr_dev = torch.full((1,), float(lr), device=self.device, dtype=torch.float32)
                 L.call("egot2_adam_step_fused_sched", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
@@ -835,3 +849,12 @@ class TranslatorEngine:
                state["v"].data_ptr(), self.arena.numel, lr, betas[0], betas[1], eps, weight_decay, int(step),
                float(grad_scale), _stream())
         self.arena.shadow_fresh = False
+
+    def grad_norm_workspace(self) -> torch.Tensor:
+        """The egot2_grad_norm workspace of this engine: zero-filled once, and every launch leaves it so.  Trainers allocate it
+        at construction, outside any CUDA-graph capture."""
+        ws = getattr(self, "_norm_ws", None)
+        if ws is None:
+            ws = self._norm_ws = torch.zeros(int(L.load().egot2_grad_norm_workspace_bytes()), device=self.device,
+                                             dtype=torch.uint8)
+        return ws

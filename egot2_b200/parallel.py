@@ -168,10 +168,13 @@ class PeerExchange:
         self.desc.off_param, self.desc.off_grad, self.desc.off_shadow, self.desc.off_flags = off_param, off_grad, off_shadow, off_flags
 
     def step(self, state, step: int, hp, stream: int, step_dev: Optional[torch.Tensor] = None, decoupled: bool = False,
-             lo: int = 0, hi: Optional[int] = None, channel: int = 0, lr_dev: Optional[torch.Tensor] = None):
+             lo: int = 0, hi: Optional[int] = None, channel: int = 0, lr_dev: Optional[torch.Tensor] = None,
+             guard: Optional[torch.Tensor] = None):
         """The exchange + optimizer step of this rank for arena elements [lo, hi) (default: everything) on flag `channel`;
         afterwards that part of the gradient arena is cleared (stream order).  lr_dev: the learning rate is read from this
-        device float when the kernel executes (optim.py), instead of hp["lr"]."""
+        device float when the kernel executes (optim.py), instead of hp["lr"].  guard: a device egot2_grad_guard - the
+        update is clipped by the global norm of the rank-averaged gradient, or skipped on every rank when it is not finite
+        (two launches); it must cover the whole arena."""
         import ctypes as C
         from . import _lib as L
         arena = self.engine.arena
@@ -186,6 +189,9 @@ class PeerExchange:
         d.lr_dev = lr_dev.data_ptr() if lr_dev is not None else None
         d.decoupled = 1 if decoupled else 0
         hi = arena.numel if hi is None else hi
+        if guard is not None and (lo, hi) != (0, arena.numel):
+            raise L.Egot2Error("PeerExchange.step: a gradient guard needs the norm of the whole arena (lo=0, hi=numel)")
+        d.guard = guard.data_ptr() if guard is not None else None
         # small exchanges: the slice owners clear the gradients in the same kernel; large ones: one local clear afterwards
         # (clearing over NVLink would double the remote traffic)
         remote_zero = (hi - lo) * 4 <= (16 << 20)

@@ -58,17 +58,40 @@ def _make_peer_exchange(engine, process_group, world):
     return peer if int(flag.item()) == 1 else None
 
 
+def _check_max_grad_norm(x) -> float:
+    x = float(x)
+    if not x > 0.0:                        # also rejects NaN
+        raise ValueError(f"max_grad_norm must be positive (math.inf: skip non-finite steps, never clip), got {x}")
+    return x
+
+
 class _OptimizerState:
-    """Learning-rate schedule and resumable optimizer state of the fused trainers.
+    """Learning-rate schedule, gradient guard and resumable optimizer state of the fused trainers.
 
     With `lr_schedule` (optim.LRSchedule) the trainer owns three device buffers: the egot2_lr_sched descriptor, the lr of
     the last step and the optimizer step count.  Every step, on every path, is egot2_opt_advance (step count + 1, lr of
     that step) followed by an optimizer launch that reads both from the device, so a replayed CUDA graph follows the
-    schedule and `set_lr_schedule` takes effect without a new capture.  Without a schedule nothing here adds a launch."""
+    schedule and `set_lr_schedule` takes effect without a new capture.
 
-    def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float):
+    With `max_grad_norm` the trainer also owns an egot2_grad_guard: right before the optimizer launch, after any gradient
+    all-reduce, egot2_grad_norm computes the global L2 norm of the gradient the optimizer would apply; the update is then
+    clipped to max_grad_norm (torch.nn.utils.clip_grad_norm_), or skipped when the norm is not finite - parameters, shadow
+    and moments unchanged, gradient cleared, the device step count taken back, so the bias corrections and the schedule
+    count applied steps only (GradScaler + LambdaLR, by contrast, advances the schedule on a skipped step).  The device
+    step count is then authoritative: only construction and load_optimizer_state_dict set it from the host.
+
+    Without either, nothing here adds a launch."""
+
+    def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float,
+                              max_grad_norm: Optional[float] = None):
         if lr_schedule is not None and lr != default_lr:
             raise ValueError("pass either lr or lr_schedule, not both")
+        self.max_grad_norm = None
+        if max_grad_norm is not None:
+            max_grad_norm = _check_max_grad_norm(max_grad_norm)
+            if os.environ.get("EGOT2_DP_SPLIT", "0") == "1":
+                raise ValueError("max_grad_norm is incompatible with EGOT2_DP_SPLIT=1: the split peer exchange updates most "
+                                 "parameters before the embedding gradients, and so the global norm, exist")
         self.lr_schedule = None
         self._epoch = 0                    # dropout epoch of the next step: the trainer advances it once per step from 0
         if not hasattr(self, "_step_dev"):
@@ -79,6 +102,11 @@ class _OptimizerState:
             self._lr_dev = torch.zeros(1, device=self.device, dtype=torch.float32)
             self.lr_schedule = lr_schedule
             self.set_lr_schedule(lr_schedule)
+        if max_grad_norm is not None:
+            self._guard_dev = torch.zeros(C.sizeof(L.GradGuard), device=self.device, dtype=torch.uint8)
+            self.engine.grad_norm_workspace()
+            self.max_grad_norm = max_grad_norm
+            self.set_max_grad_norm(max_grad_norm)
 
     def set_lr_schedule(self, schedule: LRSchedule):
         """Rewrite the device descriptor (in stream order): the next step follows `schedule` at its current step count, in
@@ -90,6 +118,41 @@ class _OptimizerState:
         # pageable source: the copy is staged before copy_ returns, so `host` may go away at once
         self._sched_dev.copy_(host, non_blocking=True)
         self.lr_schedule = schedule
+
+    def _guard_field(self, name: str, value=None, dtype=torch.float32) -> torch.Tensor:
+        """The device bytes of one egot2_grad_guard field as a 0-dim tensor view; with `value`, write it first (stream
+        order, only that field: the others belong to the kernels)."""
+        f = getattr(L.GradGuard, name)
+        view = self._guard_dev[f.offset:f.offset + f.size]
+        if value is not None:
+            host = torch.frombuffer(bytearray(bytes((C.c_float if dtype == torch.float32 else C.c_int32)(value))),
+                                    dtype=torch.uint8)
+            view.copy_(host, non_blocking=True)        # pageable source: staged before copy_ returns
+        return view.view(dtype)[0]
+
+    def set_max_grad_norm(self, max_grad_norm: float):
+        """Rewrite the guard's max_norm on the device (in stream order): the next step clips to it, in graph mode without a
+        new capture.  math.inf: skip non-finite steps, never clip."""
+        if self.max_grad_norm is None:
+            raise ValueError("this trainer was built without max_grad_norm; its optimizer launches have no gradient guard")
+        x = _check_max_grad_norm(max_grad_norm)
+        self._guard_field("max_norm", x)
+        self.max_grad_norm = x
+
+    @property
+    def last_grad_norm(self) -> torch.Tensor:
+        """The unclipped global gradient norm of the last step (what clip_grad_norm_ returns; NaN / inf on a skipped step), as
+        a 0-dim device tensor: no sync."""
+        if self.max_grad_norm is None:
+            raise ValueError("this trainer was built without max_grad_norm; no gradient norm is computed")
+        return self._guard_field("total_norm")
+
+    @property
+    def skipped_steps(self) -> torch.Tensor:
+        """The number of steps skipped for a non-finite gradient, as a 0-dim device int32 tensor: no sync."""
+        if self.max_grad_norm is None:
+            raise ValueError("this trainer was built without max_grad_norm; no step is ever skipped")
+        return self._guard_field("skipped", dtype=torch.int32)
 
     @property
     def last_lr(self) -> torch.Tensor:
@@ -104,32 +167,48 @@ class _OptimizerState:
                    stream)
 
     def _advance_eager(self) -> dict:
-        """Before an eager optimizer launch: with a schedule, advance the device step count and lr on the current stream
-        and return the launch's step_dev / lr_dev arguments; without one, nothing ({})."""
-        if self.lr_schedule is None:
+        """Before an eager optimizer launch: with a schedule or a guard, advance the device step count (and lr) on the
+        current stream and return the launch's step_dev / lr_dev / guard arguments; without either, nothing ({})."""
+        if self.lr_schedule is None and self.max_grad_norm is None:
             return {}
-        if self._step_dev_val != self.step_count - 1:
-            self._step_dev.fill_(self.step_count - 1)
-        self._opt_advance(_cur_stream(self.device))
+        if self.max_grad_norm is None and self._step_dev_val != self.step_count - 1:
+            self._step_dev.fill_(self.step_count - 1)      # with a guard the device count is authoritative (skips)
+        if self.lr_schedule is not None:
+            self._opt_advance(_cur_stream(self.device))
+        else:
+            self._step_dev.add_(1)
         self._step_dev_val = self.step_count
-        return dict(step_dev=self._step_dev, lr_dev=self._lr_dev)
+        return self._opt_args(self._step_dev)
+
+    def _opt_args(self, step_dev: torch.Tensor) -> dict:
+        """step_dev / lr_dev (/ guard) of an optimizer launch that reads the device step count."""
+        opt = dict(step_dev=step_dev, lr_dev=None if self.lr_schedule is None else self._lr_dev)
+        if self.max_grad_norm is not None:
+            opt["guard"] = self._guard_dev
+        return opt
 
     def optimizer_state_dict(self) -> dict:
         """What a run needs beyond the parameters (state_dict) to resume as if uninterrupted: the Adam moments keyed by
-        parameter name, the step count, the schedule and the dropout epoch.  Under the peer-memory exchange every rank
-        holds the moments of its own arena slice only: save and load per rank."""
+        parameter name, the step count (train_step calls), the schedule, the dropout epoch and, with a guard, max_grad_norm and
+        the number of skipped steps (read from the device: this syncs).  Under the peer-memory exchange every rank holds the
+        moments of its own arena slice only: save and load per rank."""
         arena = self.engine.arena
         zeros = None if "m" in self.opt_state else torch.zeros_like(arena.param)
         return {"step": self.step_count,
                 "exp_avg": arena.state_dict(self.opt_state.get("m", zeros)),
                 "exp_avg_sq": arena.state_dict(self.opt_state.get("v", zeros)),
                 "lr_schedule": None if self.lr_schedule is None else self.lr_schedule.to_dict(),
-                "dropout_epoch": self._epoch}
+                "dropout_epoch": self._epoch,
+                "max_grad_norm": self.max_grad_norm,
+                "skipped_steps": 0 if self.max_grad_norm is None else int(self.skipped_steps)}
 
     def load_optimizer_state_dict(self, sd: dict):
         if (sd["lr_schedule"] is None) != (self.lr_schedule is None):
             raise ValueError("optimizer state saved " + ("without" if sd["lr_schedule"] is None else "with") +
                              " an lr_schedule: build the trainer the same way")
+        if (sd.get("max_grad_norm") is None) != (self.max_grad_norm is None):
+            raise ValueError("optimizer state saved " + ("without" if sd.get("max_grad_norm") is None else "with") +
+                             " max_grad_norm: build the trainer the same way")
         arena = self.engine.arena
         for k, key in (("m", "exp_avg"), ("v", "exp_avg_sq")):
             if k in self.opt_state:        # in place: captured graphs hold these buffers
@@ -138,10 +217,14 @@ class _OptimizerState:
                 self.opt_state[k] = torch.zeros_like(arena.param)
             arena.load_state_dict(sd[key], base=self.opt_state[k])
         self.step_count = int(sd["step"])
-        self._step_dev.fill_(self.step_count)
+        skipped = int(sd.get("skipped_steps", 0))
+        self._step_dev.fill_(self.step_count - skipped)     # the device count counts applied steps
         self._step_dev_val = self.step_count
         if self.lr_schedule is not None:
             self.set_lr_schedule(LRSchedule.from_dict(sd["lr_schedule"]))
+        if self.max_grad_norm is not None:
+            self.set_max_grad_norm(sd["max_grad_norm"])
+            self._guard_field("skipped", skipped, dtype=torch.int32)
         self._epoch = int(sd["dropout_epoch"])
         if self.dropout_epoch:
             with _dev_guard(self.device):
@@ -226,7 +309,8 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
                  labels = the three (rows_i, 3) target-token tensors concatenated along rows."""
 
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
-                 ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None):
+                 ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None,
+                 max_grad_norm: Optional[float] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -256,7 +340,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 5e-4)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -333,7 +417,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
 
     def __init__(self, hidden=512, heads=8, layers=3, dropout=0.1, vocab=600, device="cuda:0", dtype: str = "bf16",
                  lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
-                 lr_schedule: Optional[LRSchedule] = None):
+                 lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -365,7 +449,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 1e-4)
+        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -448,7 +532,8 @@ def default_loss(spec: TranslatorSpec):
 class TranslatorTrainer(_OptimizerState):
     def __init__(self, spec: TranslatorSpec, device, dtype: str = "bf16", lr: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
-                 sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None):
+                 sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None,
+                 max_grad_norm: Optional[float] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -501,7 +586,7 @@ class TranslatorTrainer(_OptimizerState):
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
-        self._init_optimizer_state(lr_schedule, lr, 5e-4)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}
@@ -544,7 +629,7 @@ class TranslatorTrainer(_OptimizerState):
                 self.engine.arena.grad.zero_()
             if self.engine.dtype == "bf16" and not self.engine.arena.shadow_fresh:
                 self.engine.arena.refresh_shadow()
-            if self.graph_update and self._step_dev_val != self.step_count - 1:
+            if self.graph_update and self.max_grad_norm is None and self._step_dev_val != self.step_count - 1:
                 self._step_dev.fill_(self.step_count - 1)
             graph.replay()
             if self.graph_update:                         # the graph ended with fused Adam (+ the epoch advance)
@@ -605,7 +690,8 @@ class TranslatorTrainer(_OptimizerState):
                 self.opt_state["v"] = torch.zeros_like(self.engine.arena.param)
             if self.world > 1 and self.peer is None:      # communicator warm-up outside the capture (grad arena is zero)
                 allreduce_gradients(self.engine.arena.grad, self.pg)
-            self._step_dev.fill_(self.step_count - 1)
+            if self.max_grad_norm is None:             # with a guard the device count is authoritative (skips)
+                self._step_dev.fill_(self.step_count - 1)
             self._step_dev_val = self.step_count - 1
         if self.dp_overlap and not self.graph_update:
             torch.cuda.synchronize(self.device)
@@ -680,12 +766,10 @@ class TranslatorTrainer(_OptimizerState):
         return None if self.lr_schedule is None else self._lr_dev
 
     def _reduce_and_update(self, step_dev: Optional[torch.Tensor] = None):
-        """step_dev: the launch sits in the whole-step graph, whose side branch advances the step count (and lr)."""
+        """step_dev: the launch sits in the whole-step graph, whose side branch advances the step count (and lr).  With a
+        guard, the norm launch follows the all-reduce (engine.adam_step) or is part of the peer exchange."""
         eng = self.engine
-        if step_dev is None:
-            opt = self._advance_eager()
-        else:
-            opt = dict(step_dev=step_dev, lr_dev=self._graph_lr_dev())
+        opt = self._advance_eager() if step_dev is None else self._opt_args(step_dev)
         if self.peer is not None:                         # one kernel: reduce-scatter + Adam + all-gather over peer memory
             self.peer.step(self.opt_state, self.step_count, self.hp, torch.cuda.current_stream(self.device).cuda_stream,
                            **opt)

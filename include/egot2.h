@@ -36,6 +36,9 @@
  *                                warm-up + cosine / step-wise schedules of the HOI recipes (SURVEY.md §3.5,
  *                                HOI/optimizers/lta/lr_scheduler.py:21-26,67-91), read by egot2_adam_step_fused_sched
  *                                and by egot2_dp_reduce_adam (egot2_dp_desc.lr_dev) when they execute
+ *   egot2_grad_norm              torch.nn.utils.clip_grad_norm_ (Lightning's gradient_clip_val) and GradScaler's skip of
+ *                                non-finite steps, on the device, read by egot2_adam_step_fused_guard and by
+ *                                egot2_dp_reduce_adam (egot2_dp_desc.guard)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -431,6 +434,35 @@ int egot2_adam_step_fused_sched(float* param, float* grad, float* exp_avg, float
                                 float beta1, float beta2, float eps, float weight_decay, const int32_t* step_dev,
                                 float grad_scale, void* shadow_bf16, int32_t zero_grad, int32_t decoupled, void* stream);
 
+/* Gradient-norm clipping and skipping of non-finite steps, on the device (torch.nn.utils.clip_grad_norm_, and the step skip of
+ * torch.amp.GradScaler).  A DEVICE-resident descriptor: max_norm is the input (> 0, +inf = never clip), the rest is written by
+ * egot2_grad_norm (or by the guarded peer exchange) when it executes:
+ *   total_norm = ||grad_scale * grad||_2 over the whole arena (squares summed in fp64, fixed order: bit-reproducible);
+ *   finite total_norm:     coef = min(1, max_norm / (total_norm + 1e-6)) (fp32, clip_grad_norm_'s formula), skip = 0;
+ *   non-finite total_norm: skip = 1, ++skipped, and the optimizer step count is decremented (*step_dev, when given), so
+ *                          that it, the Adam bias corrections and the lr schedule count applied steps only. */
+typedef struct {
+  float max_norm;
+  float total_norm;
+  float coef;
+  int32_t skip;
+  int32_t skipped;
+} egot2_grad_guard;
+/* Bytes of the egot2_grad_norm workspace.  Zero-fill it once before its first use; every call leaves it that way again
+ * (its grid counter resets itself), so the call can sit in a CUDA graph. */
+size_t egot2_grad_norm_workspace_bytes(void);
+/* One launch of a fixed grid (independent of the device and of timing): per-CTA fp64 sums of squares, and the last CTA adds
+ * them in CTA order and writes total_norm / coef / skip (/ skipped, *step_dev) of *guard.  No host sync; graph-capturable. */
+int egot2_grad_norm(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev, void* workspace,
+                    size_t ws_bytes, void* stream);
+/* egot2_adam_step_fused_sched with the guard applied: the gradient is multiplied by grad_scale * guard->coef; with
+ * guard->skip the parameters, the moments and the shadow stay as they are and only the gradient is cleared (zero_grad).
+ * lr_dev NULL: the learning rate is `lr`.  decoupled = 1 runs AdamW. */
+int egot2_adam_step_fused_guard(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
+                                const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                                int32_t decoupled, const egot2_grad_guard* guard, void* stream);
+
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
  * translator gradients after backward, then the optimizer on every rank.  Here that is ONE kernel (csrc/peer.cu): gradient
@@ -457,6 +489,9 @@ typedef struct {
   int32_t zero_grads_remote;          /* 1: the owner of a slice clears that slice of every rank's gradient arena after reading
                                        * it (small arenas: no separate clear launch); 0: the caller clears its arena afterwards */
   const float* lr_dev;                /* optional: the learning rate lives on the device (egot2_opt_advance); NULL: `lr` */
+  egot2_grad_guard* guard;            /* optional: clip by the global norm of the rank-averaged gradient / skip non-finite
+                                       * steps (egot2_grad_norm's semantics; every rank reaches the same decision).  The exchange
+                                       * then runs as two launches with one more flag round trip: reduce + norm, then the update */
 } egot2_dp_desc;
 int egot2_peer_alloc(size_t bytes, void** ptr);
 int egot2_peer_free(void* ptr);
