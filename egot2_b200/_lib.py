@@ -104,11 +104,20 @@ class DpDesc(C.Structure):
     _fields_ = [("world", i32), ("rank", i32), ("numel", C.c_int64), ("slab", vp * 8), ("off_param", C.c_int64),
                 ("off_grad", C.c_int64), ("off_shadow", C.c_int64), ("off_flags", C.c_int64), ("exp_avg", vp), ("exp_avg_sq", vp),
                 ("lr", f32), ("beta1", f32), ("beta2", f32), ("eps", f32), ("weight_decay", f32), ("step", i32), ("step_dev", vp),
-                ("decoupled", i32), ("zero_grads_remote", i32), ("lr_dev", vp), ("guard", vp)]
+                ("decoupled", i32), ("zero_grads_remote", i32), ("lr_dev", vp), ("guard", vp), ("groups", vp),
+                ("block_group", vp)]
 
 
 class GradGuard(C.Structure):
     _fields_ = [("max_norm", f32), ("total_norm", f32), ("coef", f32), ("skip", i32), ("skipped", i32)]
+
+
+MAX_PARAM_GROUPS = 8
+
+
+class ParamGroups(C.Structure):
+    _fields_ = [("n_groups", i32), ("lr_mult", f32 * MAX_PARAM_GROUPS), ("weight_decay", f32 * MAX_PARAM_GROUPS),
+                ("frozen", i32 * MAX_PARAM_GROUPS)]
 
 
 class LrSched(C.Structure):
@@ -208,6 +217,9 @@ SIGNATURES = {
     "egot2_grad_norm_workspace_bytes": (sz, []),
     "egot2_grad_norm": (C.c_int, [vp, sz, f32, vp, vp, vp, sz, vp]),
     "egot2_adam_step_fused_guard": (C.c_int, [vp, vp, vp, vp, sz, f32, vp, f32, f32, f32, f32, vp, f32, vp, i32, i32, vp, vp]),
+    "egot2_adam_step_fused_groups": (C.c_int, [vp, vp, vp, vp, sz, f32, vp, f32, f32, f32, vp, f32, vp, i32, i32, vp, vp, vp,
+                                               vp]),
+    "egot2_grad_norm_groups": (C.c_int, [vp, sz, f32, vp, vp, vp, vp, vp, sz, vp]),
     "egot2_gemm": (C.c_int, [i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, i32, i32, vp]),
     "egot2_gemm_last_impl": (C.c_char_p, []),
     "egot2_layernorm_fwd": (C.c_int, [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp]),

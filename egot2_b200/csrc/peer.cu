@@ -11,7 +11,9 @@
 //      loads cross NVLink), the Adam update on the LOCAL moments, and the new parameter written as fp32 and bf16 into ALL N slabs;
 //   3. fence, tell every peer "my slice of epoch e is in your arena", and leave only when every rank said so.
 // With a gradient guard (egot2_dp_desc.guard) step 2 is split at the global norm: dp_guard_reduce_kernel, then
-// dp_guard_adam_kernel (one more flag round trip, for the per-rank partial sums of squares).
+// dp_guard_adam_kernel (one more flag round trip, for the per-rank partial sums of squares).  With parameter groups
+// (egot2_dp_desc.groups) every quad takes its group's lr and weight decay, frozen quads are neither updated nor gathered
+// (only their gradient is cleared) and stay out of the guard's norm.
 // After the kernel every rank holds bit-identical parameters (each slice is computed once, by its owner), no rank reads a
 // peer's gradients any more (so the caller may clear its gradient arena), and nothing went through the host: the kernel sits in
 // the step's CUDA graph behind the backward pass.  The message is latency-bound for the translators (0.7-9 M parameters), which
@@ -51,6 +53,8 @@ struct DpArgs {
   const float* lr_dev;                 // optional: learning rate on the device (egot2_opt_advance)
   int decoupled;
   egot2_grad_guard* guard;             // optional: global-norm clip / non-finite skip (two launches, see dp_guard_reduce_kernel)
+  const egot2_param_groups* groups;    // optional: parameter groups, with the arena's block map
+  const uint8_t* block_group;
 };
 
 __device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v) {
@@ -76,19 +80,34 @@ __device__ __forceinline__ void slice_quads(const DpArgs& a, size_t& q0, size_t&
   q0 = base + per * a.rank;
   q1 = (per * (a.rank + 1) < n4 ? per * (a.rank + 1) : n4) + base;
 }
-// the arithmetic of adam_kernel (rowops.cu), element for element
-__device__ __forceinline__ void adam_quad(const DpArgs& a, float lr, float bc1, float bc2_sqrt, const float* gg, float* w,
-                                          float* mm, float* vv) {
+// the arithmetic of adam_kernel (rowops.cu), element for element; lr and wd of the quad's parameter group (quad_hp)
+__device__ __forceinline__ void adam_quad(const DpArgs& a, float lr, float wd, float bc1, float bc2_sqrt, const float* gg,
+                                          float* w, float* mm, float* vv) {
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     float grad = gg[k];
     float wk = w[k];
-    if (a.decoupled) wk *= 1.f - lr * a.wd;
-    else if (a.wd != 0.f) grad += a.wd * wk;
+    if (a.decoupled) wk *= 1.f - lr * wd;
+    else if (wd != 0.f) grad += wd * wk;
     mm[k] = a.b1 * mm[k] + (1.f - a.b1) * grad;
     vv[k] = a.b2 * vv[k] + (1.f - a.b2) * grad * grad;
     w[k] = wk - (lr / bc1) * mm[k] / (sqrtf(vv[k]) / bc2_sqrt + a.eps);
   }
+}
+// Quad q (global, in units of 4 floats) never straddles a 64-element block: its group's lr (the step's lr times lr_mult) and
+// weight decay, and whether it is frozen.  Without groups: the step's lr, the desc's weight decay, never frozen.
+__device__ __forceinline__ bool quad_hp(const DpArgs& a, size_t q, float lr, float& lr_q, float& wd_q) {
+  lr_q = lr;
+  wd_q = a.wd;
+  if (!a.groups) return false;
+  const int k = a.block_group[q >> 4];
+  if (a.groups->frozen[k]) return true;
+  lr_q = lr * a.groups->lr_mult[k];
+  wd_q = a.groups->weight_decay[k];
+  return false;
+}
+__device__ __forceinline__ void clear_grad_quad(const DpArgs& a, size_t q) {
+  for (int p = 0; p < a.world; ++p) reinterpret_cast<float4*>(a.slab[p] + a.off_grad)[q] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 // local moments, then the all-gather: the owner writes its slice (fp32 + bf16 shadow) into every arena
 __device__ __forceinline__ void store_and_gather(const DpArgs& a, size_t q, const float* w, const float* mm, const float* vv,
@@ -180,10 +199,15 @@ __global__ void __launch_bounds__(256) dp_reduce_adam_kernel(const DpArgs a) {
     for (int u = 0; u < U; ++u) {
       const size_t q = qb + u * stride;
       if (q >= q1) continue;
+      float lr_q, wd_q;
+      if (quad_hp(a, q, lr, lr_q, wd_q)) {       // frozen: parameters, shadow and moments stay; the gradient is cleared
+        if (a.zero_remote) clear_grad_quad(a, q);
+        continue;
+      }
       float gg[4] = {g[u].x * inv_world, g[u].y * inv_world, g[u].z * inv_world, g[u].w * inv_world};
       float w[4] = {w4[u].x, w4[u].y, w4[u].z, w4[u].w};
       float mm[4] = {m4[u].x, m4[u].y, m4[u].z, m4[u].w}, vv[4] = {v4[u].x, v4[u].y, v4[u].z, v4[u].w};
-      adam_quad(a, lr, bc1, bc2_sqrt, gg, w, mm, vv);
+      adam_quad(a, lr_q, wd_q, bc1, bc2_sqrt, gg, w, mm, vv);
       store_and_gather(a, q, w, mm, vv, a.zero_remote);
     }
   }
@@ -239,7 +263,9 @@ __global__ void __launch_bounds__(256) dp_guard_reduce_kernel(const DpArgs a) {
       if (q >= q1) continue;
       const float4 gg = make_float4(g[u].x * inv_world, g[u].y * inv_world, g[u].z * inv_world, g[u].w * inv_world);
       reinterpret_cast<float4*>(a.slab[a.rank] + a.off_grad)[q] = gg;
-      s += (double)gg.x * gg.x; s += (double)gg.y * gg.y; s += (double)gg.z * gg.z; s += (double)gg.w * gg.w;
+      if (!(a.groups && a.groups->frozen[a.block_group[q >> 4]])) {      // frozen groups stay out of the norm
+        s += (double)gg.x * gg.x; s += (double)gg.y * gg.y; s += (double)gg.z * gg.z; s += (double)gg.w * gg.w;
+      }
       if (a.zero_remote)
         for (int p = 0; p < a.world; ++p)
           if (p != a.rank) reinterpret_cast<float4*>(a.slab[p] + a.off_grad)[q] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -301,13 +327,14 @@ __global__ void __launch_bounds__(256) dp_guard_adam_kernel(const DpArgs a) {
   slice_quads(a, q0, q1);
   float4* grad = reinterpret_cast<float4*>(a.slab[a.rank] + a.off_grad);
   for (size_t q = q0 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; q < q1; q += (size_t)gridDim.x * blockDim.x) {
-    if (!skip) {
+    float lr_q, wd_q;
+    if (!skip && !quad_hp(a, q, lr, lr_q, wd_q)) {
       const float4 g4 = grad[q], w4 = reinterpret_cast<const float4*>(a.slab[a.rank] + a.off_param)[q];
       const float4 m4 = reinterpret_cast<float4*>(a.m)[q], v4 = reinterpret_cast<float4*>(a.v)[q];
       float gg[4] = {g4.x * coef, g4.y * coef, g4.z * coef, g4.w * coef};
       float w[4] = {w4.x, w4.y, w4.z, w4.w};
       float mm[4] = {m4.x, m4.y, m4.z, m4.w}, vv[4] = {v4.x, v4.y, v4.z, v4.w};
-      adam_quad(a, lr, bc1, bc2_sqrt, gg, w, mm, vv);
+      adam_quad(a, lr_q, wd_q, bc1, bc2_sqrt, gg, w, mm, vv);
       store_and_gather(a, q, w, mm, vv, 0);
     }
     if (a.zero_remote) grad[q] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -384,6 +411,9 @@ static int dp_launch(const egot2_dp_desc* d, long long lo, long long hi, int cha
   a.lr_dev = d->lr_dev;
   a.decoupled = d->decoupled;
   a.guard = d->guard;
+  EGOT2_CHECK(!d->groups == !d->block_group, "dp_reduce_adam: groups and block_group go together");
+  a.groups = d->groups;
+  a.block_group = d->block_group;
   // a few CTAs per rank: the message is latency-bound, and the spinning CTAs must never crowd out other work
   const size_t per4 = ((size_t)(hi - lo) / 4 + d->world - 1) / d->world;
   // latency-bound for the small arenas (a few CTAs), bandwidth-bound for the large ones (two waves of resident CTAs)

@@ -379,14 +379,28 @@ __global__ void zero_kernel(float* p, size_t n) {
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = 0.f;
 }
 
-// DECOUPLED = torch.optim.AdamW: the weight decay scales the parameter (p *= 1 - lr*wd) instead of joining the gradient
-template <bool DECOUPLED>
+// DECOUPLED = torch.optim.AdamW: the weight decay scales the parameter (p *= 1 - lr*wd) instead of joining the gradient.
+// GROUPS: lr multiplier, weight decay and frozen flag per element from its group (egot2_param_groups).  The grid stride and
+// blockDim are multiples of 32, so a warp's 32 consecutive elements lie in one 64-element block: the map read is one broadcast
+// load per warp and iteration, and the group's values come from shared memory.
+template <bool DECOUPLED, bool GROUPS>
 __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, size_t n, float lr, float b1, float b2, float eps, float wd,
                             float bc1, float bc2_sqrt, float gscale, bf16* __restrict__ shadow, int zero_grad,
                             const int32_t* __restrict__ step_dev, const float* __restrict__ lr_dev,
-                            const egot2_grad_guard* __restrict__ guard) {
+                            const egot2_grad_guard* __restrict__ guard, const egot2_param_groups* __restrict__ groups,
+                            const uint8_t* __restrict__ block_group) {
   EGOT2_PDL_ENTER();
+  __shared__ float s_lr_mult[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1], s_wd[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1];
+  __shared__ int s_frozen[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1];
+  if (GROUPS) {
+    if (threadIdx.x < EGOT2_MAX_PARAM_GROUPS) {
+      s_lr_mult[threadIdx.x] = groups->lr_mult[threadIdx.x];
+      s_wd[threadIdx.x] = groups->weight_decay[threadIdx.x];
+      s_frozen[threadIdx.x] = groups->frozen[threadIdx.x];
+    }
+    __syncthreads();
+  }
   if (guard) {               // egot2_grad_norm ran before: clip, or skip the update and only clear the gradient
     if (guard->skip) {
       if (zero_grad)
@@ -402,15 +416,25 @@ __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float*
   }
   if (lr_dev) lr = *lr_dev;  // learning-rate schedule evaluated on the device (egot2_opt_advance)
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    float lr_e = lr, wd_e = wd;
+    if (GROUPS) {
+      const int k = block_group[i >> 6];
+      if (s_frozen[k]) {                                 // requires_grad=False: only the gradient is cleared
+        if (zero_grad) g[i] = 0.f;
+        continue;
+      }
+      lr_e = lr * s_lr_mult[k];
+      wd_e = s_wd[k];
+    }
     float grad = g[i] * gscale;
     float w = p[i];
-    if (DECOUPLED) w *= 1.f - lr * wd;
-    else if (wd != 0.f) grad += wd * w;
+    if (DECOUPLED) w *= 1.f - lr_e * wd_e;
+    else if (wd_e != 0.f) grad += wd_e * w;
     const float mi = b1 * m[i] + (1.f - b1) * grad;
     const float vi = b2 * v[i] + (1.f - b2) * grad * grad;
     m[i] = mi; v[i] = vi;
     // torch.optim.Adam: denom = sqrt(v)/sqrt(bias_correction2) + eps ; step = lr / bias_correction1
-    const float wn = w - (lr / bc1) * mi / (sqrtf(vi) / bc2_sqrt + eps);
+    const float wn = w - (lr_e / bc1) * mi / (sqrtf(vi) / bc2_sqrt + eps);
     p[i] = wn;
     if (shadow) shadow[i] = __float2bfloat16_rn(wn);     // the bf16 copy the next forward's GEMMs read
     if (zero_grad) g[i] = 0.f;                           // the next backward accumulates into a clean arena
@@ -448,13 +472,23 @@ __global__ void opt_advance_kernel(int32_t* __restrict__ step, const egot2_lr_sc
 
 // egot2_grad_norm: a fixed grid (not sm_count-dependent, so every GPU adds in the same order), fp64 squares per thread in
 // index order, a fixed-order CTA sum, and the last CTA to finish adds the per-CTA sums in CTA order.
+// GROUPS: the elements of frozen groups count as 0 (a quad never straddles a 64-element block), so the order of the sum is
+// that of the ungrouped kernel over the same gradient with the frozen part cleared.
 constexpr int kNormCtas = 512, kNormThreads = 256;
+template <bool GROUPS>
 __global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const float* __restrict__ g, size_t n, float scale,
                                                                  egot2_grad_guard* __restrict__ guard, int32_t* step_dev,
-                                                                 double* part, unsigned int* ctr) {
+                                                                 double* part, unsigned int* ctr,
+                                                                 const egot2_param_groups* __restrict__ groups,
+                                                                 const uint8_t* __restrict__ block_group) {
   EGOT2_PDL_ENTER();
   __shared__ double sh[kNormThreads / 32];
   __shared__ unsigned int s_last;
+  __shared__ int s_frozen[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1];
+  if (GROUPS) {
+    if (threadIdx.x < EGOT2_MAX_PARAM_GROUPS) s_frozen[threadIdx.x] = groups->frozen[threadIdx.x];
+    __syncthreads();
+  }
   const size_t tid = blockIdx.x * (size_t)kNormThreads + threadIdx.x, stride = (size_t)kNormCtas * kNormThreads;
   double s = 0.0;
   size_t tail = 0;
@@ -465,7 +499,10 @@ __global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const float* __
     for (size_t q = tid; q < n4; q += stride * U) {
       float4 x[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u) x[u] = q + u * stride < n4 ? g4[q + u * stride] : make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int u = 0; u < U; ++u) {
+        const size_t qu = q + u * stride;
+        x[u] = qu < n4 && !(GROUPS && s_frozen[block_group[qu >> 4]]) ? g4[qu] : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         s += (double)x[u].x * x[u].x; s += (double)x[u].y * x[u].y;
@@ -474,7 +511,8 @@ __global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const float* __
     }
     tail = n4 * 4;
   }
-  for (size_t i = tail + tid; i < n; i += stride) s += (double)g[i] * g[i];
+  for (size_t i = tail + tid; i < n; i += stride)
+    if (!(GROUPS && s_frozen[block_group[i >> 6]])) s += (double)g[i] * g[i];
   s = block_sum_f64(s, sh);
   if (threadIdx.x == 0) {
     part[blockIdx.x] = s;
@@ -1078,18 +1116,18 @@ extern "C" int egot2_cast_bf16_to_f32(const void* src, float* dst, size_t n, voi
 static int adam_launch(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr, float beta1,
                        float beta2, float eps, float weight_decay, int32_t step, float grad_scale, void* shadow,
                        int zero_grad, void* stream, const int32_t* step_dev = nullptr, bool decoupled = false,
-                       const float* lr_dev = nullptr, const egot2_grad_guard* guard = nullptr) {
+                       const float* lr_dev = nullptr, const egot2_grad_guard* guard = nullptr,
+                       const egot2_param_groups* groups = nullptr, const uint8_t* block_group = nullptr) {
   EGOT2_CHECK(step >= 1 || step_dev, "adam: step must be >= 1");
   if (n == 0) return 0;
   const float bc1 = 1.f - powf(beta1, (float)step);
   const float bc2 = 1.f - powf(beta2, (float)step);
-  ProfScope prof((cudaStream_t)stream, "adam n%zu", n);
-  if (decoupled)
-    launch(adam_kernel<true>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev, guard);
-  else
-    launch(adam_kernel<false>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr,
-           beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev, guard);
+  ProfScope prof((cudaStream_t)stream, groups ? "adam_groups n%zu" : "adam n%zu", n);
+  auto* kernel = groups ? (decoupled ? adam_kernel<true, true> : adam_kernel<false, true>)
+                        : (decoupled ? adam_kernel<true, false> : adam_kernel<false, false>);
+  launch(kernel, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
+         eps, weight_decay, bc1, sqrtf(bc2), grad_scale, (bf16*)shadow, zero_grad, step_dev, lr_dev, guard, groups,
+         block_group);
   EGOT2_LAUNCH_CHECK();
   return 0;
 }
@@ -1141,20 +1179,42 @@ extern "C" int egot2_adam_step_fused_guard(float* param, float* grad, float* exp
                      zero_grad, stream, step_dev, decoupled != 0, lr_dev, guard);
 }
 
+extern "C" int egot2_adam_step_fused_groups(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
+                                            const float* lr_dev, float beta1, float beta2, float eps,
+                                            const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                                            int32_t decoupled, const egot2_grad_guard* guard,
+                                            const egot2_param_groups* groups, const uint8_t* block_group, void* stream) {
+  EGOT2_CHECK(step_dev != nullptr && groups != nullptr && (block_group != nullptr || n == 0),
+              "adam: step_dev / groups / block_group is null");
+  return adam_launch(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, 0.f, 1, grad_scale, shadow_bf16, zero_grad,
+                     stream, step_dev, decoupled != 0, lr_dev, guard, groups, block_group);
+}
+
 extern "C" size_t egot2_grad_norm_workspace_bytes(void) { return kNormCtas * sizeof(double) + 16; }
 
-extern "C" int egot2_grad_norm(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev,
-                               void* workspace, size_t ws_bytes, void* stream) {
+static int grad_norm_launch(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev,
+                            const egot2_param_groups* groups, const uint8_t* block_group, void* workspace, size_t ws_bytes,
+                            void* stream) {
   EGOT2_CHECK(guard && workspace && (grad || n == 0), "grad_norm: grad / guard / workspace is null");
   EGOT2_CHECK(ws_bytes >= egot2_grad_norm_workspace_bytes() && reinterpret_cast<uintptr_t>(workspace) % 8 == 0,
               "grad_norm: workspace of %zu bytes (8-byte aligned) needed, got %zu", egot2_grad_norm_workspace_bytes(), ws_bytes);
   double* part = (double*)workspace;
   unsigned int* ctr = (unsigned int*)(part + kNormCtas);
-  ProfScope prof((cudaStream_t)stream, "grad_norm n%zu", n);
-  launch(grad_norm_kernel, dim3(kNormCtas), dim3(kNormThreads), 0, (cudaStream_t)stream, grad, n, grad_scale, guard, step_dev,
-         part, ctr);
+  ProfScope prof((cudaStream_t)stream, groups ? "grad_norm_groups n%zu" : "grad_norm n%zu", n);
+  launch(groups ? grad_norm_kernel<true> : grad_norm_kernel<false>, dim3(kNormCtas), dim3(kNormThreads), 0,
+         (cudaStream_t)stream, grad, n, grad_scale, guard, step_dev, part, ctr, groups, block_group);
   EGOT2_LAUNCH_CHECK();
   return 0;
+}
+extern "C" int egot2_grad_norm(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev,
+                               void* workspace, size_t ws_bytes, void* stream) {
+  return grad_norm_launch(grad, n, grad_scale, guard, step_dev, nullptr, nullptr, workspace, ws_bytes, stream);
+}
+extern "C" int egot2_grad_norm_groups(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard,
+                                      int32_t* step_dev, const egot2_param_groups* groups, const uint8_t* block_group,
+                                      void* workspace, size_t ws_bytes, void* stream) {
+  EGOT2_CHECK(groups != nullptr && (block_group != nullptr || n == 0), "grad_norm: groups / block_group is null");
+  return grad_norm_launch(grad, n, grad_scale, guard, step_dev, groups, block_group, workspace, ws_bytes, stream);
 }
 
 extern "C" int egot2_opt_advance(int32_t* step_dev, const egot2_lr_sched* sched, float* lr_dev, void* stream) {

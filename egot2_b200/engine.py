@@ -791,7 +791,7 @@ class TranslatorEngine:
     def adam_step(self, state: Dict[str, torch.Tensor], step: int, lr: float = 5e-4, betas=(0.9, 0.999),
                   eps: float = 1e-8, weight_decay: float = 0.0, grad_scale: float = 1.0, fused: bool = False,
                   step_dev: Optional[torch.Tensor] = None, decoupled: bool = False, lr_dev: Optional[torch.Tensor] = None,
-                  guard: Optional[torch.Tensor] = None):
+                  guard: Optional[torch.Tensor] = None, groups: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
         """torch.optim.Adam over the whole arena in one launch (HHI/tasks/ttm/video_task.py:64-66: lr 5e-4).
         fused: the same launch also writes the bf16 shadow of the updated parameters (bf16 engines) and clears the
         gradient arena, so the next step needs neither the cast launch nor a fill (callers then pass
@@ -800,7 +800,10 @@ class TranslatorEngine:
         kernel executes (graph replays, device-evaluated schedules: optim.py); lr_dev needs step_dev.
         guard: a device egot2_grad_guard (_lib.GradGuard bytes; fused, needs step_dev): egot2_grad_norm of grad_scale * the
         gradient arena first, then the update clipped by that norm, or skipped (gradient cleared, step count taken back)
-        when it is not finite."""
+        when it is not finite.
+        groups: (device egot2_param_groups bytes, uint8 map of one group per 64-element block) - torch.optim param groups over
+        the arena (fused, needs step_dev): every element takes its group's lr multiplier, weight decay (`weight_decay` is
+        unused) and frozen flag, still in one launch; with a guard the norm leaves frozen groups out."""
         if "m" not in state:
             state["m"] = torch.zeros_like(self.arena.param)
             state["v"] = torch.zeros_like(self.arena.param)
@@ -808,13 +811,27 @@ class TranslatorEngine:
             raise L.Egot2Error("adam_step: lr_dev needs step_dev (egot2_opt_advance keeps both on the device)")
         if guard is not None and (step_dev is None or not fused):
             raise L.Egot2Error("adam_step: a gradient guard needs the fused launch and step_dev (a skip takes the step back)")
+        if groups is not None and (step_dev is None or not fused):
+            raise L.Egot2Error("adam_step: parameter groups need the fused launch and step_dev")
         if fused:
             shadow = None
             if self.dtype == "bf16":
                 if self.arena.shadow is None:
                     self.arena.refresh_shadow()
                 shadow = self.arena.shadow.data_ptr()
-            if guard is not None:
+            if groups is not None:
+                desc, block_group = groups
+                if guard is not None:
+                    ws = self.grad_norm_workspace()
+                    L.call("egot2_grad_norm_groups", self.arena.grad.data_ptr(), self.arena.numel, float(grad_scale),
+                           guard.data_ptr(), step_dev.data_ptr(), desc.data_ptr(), block_group.data_ptr(), ws.data_ptr(),
+                           ws.numel(), _stream())
+                L.call("egot2_adam_step_fused_groups", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
+                       state["m"].data_ptr(), state["v"].data_ptr(), self.arena.numel, float(lr),
+                       None if lr_dev is None else lr_dev.data_ptr(), betas[0], betas[1], eps, step_dev.data_ptr(),
+                       float(grad_scale), shadow, 1, 1 if decoupled else 0, None if guard is None else guard.data_ptr(),
+                       desc.data_ptr(), block_group.data_ptr(), _stream())
+            elif guard is not None:
                 ws = self.grad_norm_workspace()
                 L.call("egot2_grad_norm", self.arena.grad.data_ptr(), self.arena.numel, float(grad_scale), guard.data_ptr(),
                        step_dev.data_ptr(), ws.data_ptr(), ws.numel(), _stream())

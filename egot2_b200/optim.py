@@ -9,12 +9,20 @@ deliberately does not evaluate the schedule (the only host restatement of lr_at 
 The policies are the SlowFast-style ones the HOI configs select (SURVEY.md §2.2, §3.5: Adam + warm-up cosine,
 HOI/optimizers/lta/lr_scheduler.py:21-26,67-91): 'constant', 'cosine' (with end_lr), 'steps' (steps with relative lrs), each
 with an optional linear warm-up.  Steps are optimizer steps; callers that think in epochs convert.
+
+`ParamGroup` is the fused trainers' form of torch.optim's param groups (per-group weight decay and lr multiplier, frozen
+parameters).  They are applied per element by the optimizer kernels, from a device-resident `egot2_param_groups` descriptor
+and a map of one group per 64-element block of the parameter arena (include/egot2.h); `resolve_param_groups` builds both.
 """
 from __future__ import annotations
 
 import dataclasses
+import fnmatch
+import math
 from dataclasses import dataclass
-from typing import Sequence, Tuple
+from typing import Dict, Mapping, Optional, Sequence, Tuple
+
+import numpy as np
 
 from . import _lib as L
 
@@ -85,3 +93,75 @@ class LRSchedule:
     @classmethod
     def from_dict(cls, d: dict) -> "LRSchedule":
         return cls(**{**d, "milestones": tuple(d["milestones"]), "factors": tuple(d["factors"])})
+
+
+def check_group_hp(name: str, x: float) -> float:
+    x = float(x)
+    if not (math.isfinite(x) and x >= 0.0):
+        raise ValueError(f"ParamGroup: {name} must be finite and >= 0, got {x}")
+    return x
+
+
+@dataclass(frozen=True)
+class ParamGroup:
+    """One optimizer parameter group of a fused trainer (trainer.py): the parameters whose reference state_dict names
+    (spec.param_shapes() keys) match one of `patterns` (fnmatch).  Their lr is the trainer's lr (fixed or scheduled) times
+    lr_mult; weight_decay None inherits the trainer's; frozen is requires_grad=False (parameters and moments stay as they
+    are, and the gradient stays out of the max_grad_norm norm).  A parameter joins the first group that matches it;
+    unmatched parameters form group 0 with lr_mult 1 and the trainer's weight_decay."""
+    patterns: Tuple[str, ...]
+    lr_mult: float = 1.0
+    weight_decay: Optional[float] = None
+    frozen: bool = False
+
+    def __post_init__(self):
+        pats = (self.patterns,) if isinstance(self.patterns, str) else tuple(self.patterns)
+        if not pats or not all(isinstance(p, str) for p in pats):
+            raise ValueError(f"ParamGroup: patterns must be one or more strings, got {self.patterns!r}")
+        object.__setattr__(self, "patterns", pats)
+        object.__setattr__(self, "lr_mult", check_group_hp("lr_mult", self.lr_mult))
+        if self.weight_decay is not None:
+            object.__setattr__(self, "weight_decay", check_group_hp("weight_decay", self.weight_decay))
+        object.__setattr__(self, "frozen", bool(self.frozen))
+
+
+def resolve_param_groups(groups: Sequence[ParamGroup], shapes: Mapping[str, Tuple[int, ...]], offsets: Mapping[str, int],
+                         numel: int, block: int = 64) -> np.ndarray:
+    """The uint8 map of one group per `block`-element block of an arena of `numel` elements with these offsets: a parameter's
+    group is the first ParamGroup with a pattern that matches its name.  Group 0 is the default group, groups[i] is group
+    i + 1.  Raises ValueError for a pattern that matches nothing, more than MAX_PARAM_GROUPS groups, or two parameters of
+    different groups in one block."""
+    if len(groups) + 1 > L.MAX_PARAM_GROUPS:
+        raise ValueError(f"at most {L.MAX_PARAM_GROUPS} parameter groups, the default group included: got {len(groups) + 1}")
+    names = list(shapes)
+    for g in groups:
+        for pat in g.patterns:
+            if not fnmatch.filter(names, pat):
+                raise ValueError(f"ParamGroup pattern {pat!r} matches no parameter")
+    index = []
+    for n in names:
+        index.append(next((i + 1 for i, g in enumerate(groups) if any(fnmatch.fnmatchcase(n, p) for p in g.patterns)), 0))
+    group_of = dict(zip(names, index))
+    bmap = np.zeros((numel + block - 1) // block, dtype=np.uint8)
+    edge: Dict[int, str] = {}                 # first / last block of a parameter -> the parameter that claimed it
+    for n, k in zip(names, index):
+        size = int(np.prod(shapes[n], dtype=np.int64))
+        if size == 0:
+            continue
+        b0, b1 = offsets[n] // block, (offsets[n] + size - 1) // block
+        for b in {b0, b1}:                     # only a first or last block can be shared (parameters do not overlap)
+            other = edge.setdefault(b, n)
+            if group_of[other] != k:
+                raise ValueError(f"parameters {other!r} (group {group_of[other]}) and {n!r} (group {k}) share a "
+                                 f"{block}-element block of the arena and must be in the same parameter group")
+        bmap[b0:b1 + 1] = k
+    return bmap
+
+
+def pack_param_groups(hp: Sequence[Tuple[float, float, bool]]) -> L.ParamGroups:
+    """The egot2_param_groups of (lr_mult, weight_decay, frozen) per group."""
+    d = L.ParamGroups()
+    d.n_groups = len(hp)
+    for i, (lr_mult, wd, frozen) in enumerate(hp):
+        d.lr_mult[i], d.weight_decay[i], d.frozen[i] = lr_mult, wd, int(frozen)
+    return d

@@ -169,12 +169,13 @@ class PeerExchange:
 
     def step(self, state, step: int, hp, stream: int, step_dev: Optional[torch.Tensor] = None, decoupled: bool = False,
              lo: int = 0, hi: Optional[int] = None, channel: int = 0, lr_dev: Optional[torch.Tensor] = None,
-             guard: Optional[torch.Tensor] = None):
+             guard: Optional[torch.Tensor] = None, groups: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
         """The exchange + optimizer step of this rank for arena elements [lo, hi) (default: everything) on flag `channel`;
         afterwards that part of the gradient arena is cleared (stream order).  lr_dev: the learning rate is read from this
         device float when the kernel executes (optim.py), instead of hp["lr"].  guard: a device egot2_grad_guard - the
         update is clipped by the global norm of the rank-averaged gradient, or skipped on every rank when it is not finite
-        (two launches); it must cover the whole arena."""
+        (two launches); it must cover the whole arena.  groups: (device egot2_param_groups, block map of the whole arena), as
+        in engine.adam_step; hp["weight_decay"] is then unused."""
         import ctypes as C
         from . import _lib as L
         arena = self.engine.arena
@@ -192,6 +193,7 @@ class PeerExchange:
         if guard is not None and (lo, hi) != (0, arena.numel):
             raise L.Egot2Error("PeerExchange.step: a gradient guard needs the norm of the whole arena (lo=0, hi=numel)")
         d.guard = guard.data_ptr() if guard is not None else None
+        d.groups, d.block_group = (None, None) if groups is None else (groups[0].data_ptr(), groups[1].data_ptr())
         # small exchanges: the slice owners clear the gradients in the same kernel; large ones: one local clear afterwards
         # (clearing over NVLink would double the remote traffic)
         remote_zero = (hi - lo) * 4 <= (16 << 20)

@@ -18,8 +18,8 @@ import os
 import torch
 
 from . import _lib as L
-from .engine import Activations, TranslatorEngine
-from .optim import LRSchedule
+from .engine import _ALIGN, Activations, TranslatorEngine
+from .optim import LRSchedule, ParamGroup, check_group_hp, pack_param_groups, resolve_param_groups
 from .parallel import allreduce_gradients
 from .specs import TranslatorSpec
 
@@ -80,10 +80,18 @@ class _OptimizerState:
     count applied steps only (GradScaler + LambdaLR, by contrast, advances the schedule on a skipped step).  The device
     step count is then authoritative: only construction and load_optimizer_state_dict set it from the host.
 
-    Without either, nothing here adds a launch."""
+    With `param_groups` (optim.ParamGroup) the trainer owns an egot2_param_groups descriptor and a map of one group per
+    64-element arena block; the optimizer launch (and the guard's norm) read both, so per-group weight decay, lr multipliers
+    and frozen parameters cost no launch of their own, and `set_param_group` takes effect without a new capture.  The
+    optimizer launch then always reads the device step count.  Membership and `frozen` are fixed at construction: unfreezing
+    a group later would need a step count per group, since torch starts the bias correction of parameters that first get
+    optimizer state late from step 1.
+
+    Without any of them, nothing here adds a launch."""
 
     def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float,
-                              max_grad_norm: Optional[float] = None):
+                              max_grad_norm: Optional[float] = None,
+                              param_groups: Optional[Sequence[ParamGroup]] = None):
         if lr_schedule is not None and lr != default_lr:
             raise ValueError("pass either lr or lr_schedule, not both")
         self.max_grad_norm = None
@@ -107,6 +115,37 @@ class _OptimizerState:
             self.engine.grad_norm_workspace()
             self.max_grad_norm = max_grad_norm
             self.set_max_grad_norm(max_grad_norm)
+        self.param_groups = None
+        self._groups = None
+        if param_groups is not None:
+            param_groups = list(param_groups)
+            arena = self.engine.arena
+            bmap = resolve_param_groups(param_groups, arena.shapes, arena.offsets, arena.numel, _ALIGN)
+            self.param_groups = param_groups
+            wd = self.hp["weight_decay"]
+            # (lr_mult, weight_decay, frozen) of group 0 (unmatched parameters) and of every ParamGroup, as on the device
+            self._group_hp = [(1.0, float(wd), False)] + [
+                (g.lr_mult, float(wd) if g.weight_decay is None else g.weight_decay, g.frozen) for g in param_groups]
+            self._groups = (torch.zeros(C.sizeof(L.ParamGroups), device=self.device, dtype=torch.uint8),
+                            torch.from_numpy(bmap).to(self.device))
+            self._write_param_groups()
+
+    def _write_param_groups(self):
+        host = torch.frombuffer(bytearray(bytes(pack_param_groups(self._group_hp))), dtype=torch.uint8)
+        self._groups[0].copy_(host, non_blocking=True)          # pageable source: staged before copy_ returns
+
+    def set_param_group(self, index: int, lr_mult: Optional[float] = None, weight_decay: Optional[float] = None):
+        """Change the lr multiplier and / or weight decay of parameter group `index` (0: the parameters no ParamGroup matched,
+        i: param_groups[i - 1]) on the device, in stream order: the next step uses them, in graph mode without a new
+        capture.  Membership and `frozen` are fixed at construction."""
+        if self.param_groups is None:
+            raise ValueError("this trainer was built without param_groups")
+        if not 0 <= index < len(self._group_hp):
+            raise ValueError(f"no parameter group {index}: the trainer has {len(self._group_hp)} (0 = the default group)")
+        old_lr_mult, old_wd, frozen = self._group_hp[index]
+        self._group_hp[index] = (old_lr_mult if lr_mult is None else check_group_hp("lr_mult", lr_mult),
+                                 old_wd if weight_decay is None else check_group_hp("weight_decay", weight_decay), frozen)
+        self._write_param_groups()
 
     def set_lr_schedule(self, schedule: LRSchedule):
         """Rewrite the device descriptor (in stream order): the next step follows `schedule` at its current step count, in
@@ -167,9 +206,10 @@ class _OptimizerState:
                    stream)
 
     def _advance_eager(self) -> dict:
-        """Before an eager optimizer launch: with a schedule or a guard, advance the device step count (and lr) on the
-        current stream and return the launch's step_dev / lr_dev / guard arguments; without either, nothing ({})."""
-        if self.lr_schedule is None and self.max_grad_norm is None:
+        """Before an eager optimizer launch: with a schedule, a guard or parameter groups, advance the device step count (and
+        lr) on the current stream and return the launch's step_dev / lr_dev / guard / groups arguments; without any, nothing
+        ({})."""
+        if self.lr_schedule is None and self.max_grad_norm is None and self._groups is None:
             return {}
         if self.max_grad_norm is None and self._step_dev_val != self.step_count - 1:
             self._step_dev.fill_(self.step_count - 1)      # with a guard the device count is authoritative (skips)
@@ -181,16 +221,19 @@ class _OptimizerState:
         return self._opt_args(self._step_dev)
 
     def _opt_args(self, step_dev: torch.Tensor) -> dict:
-        """step_dev / lr_dev (/ guard) of an optimizer launch that reads the device step count."""
+        """step_dev / lr_dev (/ guard / groups) of an optimizer launch that reads the device step count."""
         opt = dict(step_dev=step_dev, lr_dev=None if self.lr_schedule is None else self._lr_dev)
         if self.max_grad_norm is not None:
             opt["guard"] = self._guard_dev
+        if self._groups is not None:
+            opt["groups"] = self._groups
         return opt
 
     def optimizer_state_dict(self) -> dict:
         """What a run needs beyond the parameters (state_dict) to resume as if uninterrupted: the Adam moments keyed by
         parameter name, the step count (train_step calls), the schedule, the dropout epoch and, with a guard, max_grad_norm and
-        the number of skipped steps (read from the device: this syncs).  Under the peer-memory exchange every rank holds the
+        the number of skipped steps (read from the device: this syncs), and with parameter groups every group's patterns,
+        frozen flag and current lr_mult / weight_decay (group 0 first).  Under the peer-memory exchange every rank holds the
         moments of its own arena slice only: save and load per rank."""
         arena = self.engine.arena
         zeros = None if "m" in self.opt_state else torch.zeros_like(arena.param)
@@ -200,7 +243,13 @@ class _OptimizerState:
                 "lr_schedule": None if self.lr_schedule is None else self.lr_schedule.to_dict(),
                 "dropout_epoch": self._epoch,
                 "max_grad_norm": self.max_grad_norm,
-                "skipped_steps": 0 if self.max_grad_norm is None else int(self.skipped_steps)}
+                "skipped_steps": 0 if self.max_grad_norm is None else int(self.skipped_steps),
+                "param_groups": None if self.param_groups is None else self._groups_state()}
+
+    def _groups_state(self) -> List[dict]:
+        pats = [None] + [list(g.patterns) for g in self.param_groups]
+        return [dict(patterns=p, lr_mult=lr_mult, weight_decay=wd, frozen=frozen)
+                for p, (lr_mult, wd, frozen) in zip(pats, self._group_hp)]
 
     def load_optimizer_state_dict(self, sd: dict):
         if (sd["lr_schedule"] is None) != (self.lr_schedule is None):
@@ -209,6 +258,13 @@ class _OptimizerState:
         if (sd.get("max_grad_norm") is None) != (self.max_grad_norm is None):
             raise ValueError("optimizer state saved " + ("without" if sd.get("max_grad_norm") is None else "with") +
                              " max_grad_norm: build the trainer the same way")
+        saved_groups = sd.get("param_groups")
+        if saved_groups is not None or self.param_groups is not None:
+            def membership(gs):
+                return None if gs is None else [(g["patterns"], g["frozen"]) for g in gs]
+            if membership(saved_groups) != membership(None if self.param_groups is None else self._groups_state()):
+                raise ValueError("optimizer state saved with other parameter groups (patterns / frozen): build the trainer "
+                                 "with the same param_groups")
         arena = self.engine.arena
         for k, key in (("m", "exp_avg"), ("v", "exp_avg_sq")):
             if k in self.opt_state:        # in place: captured graphs hold these buffers
@@ -225,6 +281,9 @@ class _OptimizerState:
         if self.max_grad_norm is not None:
             self.set_max_grad_norm(sd["max_grad_norm"])
             self._guard_field("skipped", skipped, dtype=torch.int32)
+        if saved_groups is not None:
+            for i, g in enumerate(saved_groups):
+                self.set_param_group(i, lr_mult=g["lr_mult"], weight_decay=g["weight_decay"])
         self._epoch = int(sd["dropout_epoch"])
         if self.dropout_epoch:
             with _dev_guard(self.device):
@@ -310,7 +369,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
 
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
                  ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None,
-                 max_grad_norm: Optional[float] = None):
+                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -340,7 +399,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -417,7 +476,8 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
 
     def __init__(self, hidden=512, heads=8, layers=3, dropout=0.1, vocab=600, device="cuda:0", dtype: str = "bf16",
                  lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
-                 lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None):
+                 lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None,
+                 param_groups: Optional[Sequence[ParamGroup]] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -449,7 +509,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm)
+        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -533,7 +593,7 @@ class TranslatorTrainer(_OptimizerState):
     def __init__(self, spec: TranslatorSpec, device, dtype: str = "bf16", lr: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
                  sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None,
-                 max_grad_norm: Optional[float] = None):
+                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -586,7 +646,7 @@ class TranslatorTrainer(_OptimizerState):
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}
@@ -725,13 +785,14 @@ class TranslatorTrainer(_OptimizerState):
                 self._peer_stream.wait_stream(cur)
                 with torch.cuda.stream(self._peer_stream):
                     self.peer.step(self.opt_state, self.step_count, self.hp, self._peer_stream.cuda_stream,
-                                   step_dev=self._step_dev, lo=nb, hi=n, channel=0, lr_dev=self._graph_lr_dev())
+                                   step_dev=self._step_dev, lo=nb, hi=n, channel=0, lr_dev=self._graph_lr_dev(),
+                                   groups=self._groups)
                 self.engine.backward(act, zero_grad=False, stage="embed")
                 self._bump_stream.wait_stream(cur)
                 with torch.cuda.stream(self._bump_stream):
                     self._advance_epoch()
                 self.peer.step(self.opt_state, self.step_count, self.hp, cur.cuda_stream, step_dev=self._step_dev,
-                               lo=0, hi=nb, channel=1, lr_dev=self._graph_lr_dev())
+                               lo=0, hi=nb, channel=1, lr_dev=self._graph_lr_dev(), groups=self._groups)
                 cur.wait_stream(self._peer_stream)
                 cur.wait_stream(self._bump_stream)
                 self._grad_clean = True

@@ -39,6 +39,8 @@
  *   egot2_grad_norm              torch.nn.utils.clip_grad_norm_ (Lightning's gradient_clip_val) and GradScaler's skip of
  *                                non-finite steps, on the device, read by egot2_adam_step_fused_guard and by
  *                                egot2_dp_reduce_adam (egot2_dp_desc.guard)
+ *   egot2_adam_step_fused_groups torch.optim param groups (per-group weight decay / lr multiplier, frozen parameters) over the
+ *                                flat arena in the same one launch (SlowFast's construct_optimizer, HOI/optimizers/)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -463,6 +465,36 @@ int egot2_adam_step_fused_guard(float* param, float* grad, float* exp_avg, float
                                 const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
                                 int32_t decoupled, const egot2_grad_guard* guard, void* stream);
 
+/* Parameter groups (torch.optim param groups: per-group weight decay and lr multiplier, and frozen parameters), on the device.
+ * A DEVICE-resident descriptor plus a DEVICE map block_group[ceil(n / 64)]: element i belongs to group block_group[i / 64]
+ * (< n_groups).  For the elements of group k, with lr the step's learning rate (by value or from lr_dev):
+ *   Adam:   grad += weight_decay[k] * param;                  AdamW: param *= 1 - lr * lr_mult[k] * weight_decay[k];
+ *   the step size is lr * lr_mult[k] (lr_mult[k] = 0 still updates the moments, as torch does with lr = 0);
+ *   frozen[k] != 0 (requires_grad=False): parameters, shadow and moments are left as they are, the gradient is only cleared
+ *   (zero_grad), and egot2_grad_norm_groups leaves it out of the norm.
+ * The descriptor is read when a kernel executes, so a CUDA graph follows a descriptor rewritten between replays. */
+#define EGOT2_MAX_PARAM_GROUPS 8
+typedef struct {
+  int32_t n_groups;                     /* 1..EGOT2_MAX_PARAM_GROUPS */
+  float lr_mult[8];
+  float weight_decay[8];
+  int32_t frozen[8];
+} egot2_param_groups;
+/* egot2_adam_step_fused_guard with parameter groups: every element takes its group's lr multiplier, weight decay and frozen
+ * flag (there is no arena-wide weight_decay argument).  lr_dev NULL: the learning rate is `lr`; guard NULL: no clipping or
+ * skipping (with a guard, egot2_grad_norm_groups runs first).  step_dev is required.  decoupled = 1 runs AdamW. */
+int egot2_adam_step_fused_groups(float* param, float* grad, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
+                                 const float* lr_dev, float beta1, float beta2, float eps, const int32_t* step_dev,
+                                 float grad_scale, void* shadow_bf16, int32_t zero_grad, int32_t decoupled,
+                                 const egot2_grad_guard* guard, const egot2_param_groups* groups,
+                                 const uint8_t* block_group, void* stream);
+/* egot2_grad_norm over the elements of non-frozen groups only (clip_grad_norm_ over the trainable parameters): a NaN / inf in
+ * a frozen gradient neither clips nor skips.  Same fixed grid and summation order as egot2_grad_norm, with frozen elements
+ * counted as 0. */
+int egot2_grad_norm_groups(const float* grad, size_t n, float grad_scale, egot2_grad_guard* guard, int32_t* step_dev,
+                           const egot2_param_groups* groups, const uint8_t* block_group, void* workspace, size_t ws_bytes,
+                           void* stream);
+
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
  * translator gradients after backward, then the optimizer on every rank.  Here that is ONE kernel (csrc/peer.cu): gradient
@@ -492,6 +524,9 @@ typedef struct {
   egot2_grad_guard* guard;            /* optional: clip by the global norm of the rank-averaged gradient / skip non-finite
                                        * steps (egot2_grad_norm's semantics; every rank reaches the same decision).  The exchange
                                        * then runs as two launches with one more flag round trip: reduce + norm, then the update */
+  const egot2_param_groups* groups;   /* optional, with block_group: parameter groups (egot2_adam_step_fused_groups' semantics;
+                                       * `weight_decay` above is then unused, and the guard's norm leaves frozen groups out) */
+  const uint8_t* block_group;         /* the group of every 64-element block of the WHOLE arena (also for a [lo, hi) range) */
 } egot2_dp_desc;
 int egot2_peer_alloc(size_t bytes, void** ptr);
 int egot2_peer_free(void* ptr);
