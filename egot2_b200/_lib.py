@@ -105,7 +105,7 @@ class DpDesc(C.Structure):
                 ("off_grad", C.c_int64), ("off_shadow", C.c_int64), ("off_flags", C.c_int64), ("exp_avg", vp), ("exp_avg_sq", vp),
                 ("lr", f32), ("beta1", f32), ("beta2", f32), ("eps", f32), ("weight_decay", f32), ("step", i32), ("step_dev", vp),
                 ("decoupled", i32), ("zero_grads_remote", i32), ("lr_dev", vp), ("guard", vp), ("groups", vp),
-                ("block_group", vp)]
+                ("block_group", vp), ("sgd", i32), ("momentum", f32), ("dampening", f32), ("nesterov", i32)]
 
 
 class GradGuard(C.Structure):
@@ -220,6 +220,7 @@ SIGNATURES = {
     "egot2_adam_step_fused_groups": (C.c_int, [vp, vp, vp, vp, sz, f32, vp, f32, f32, f32, vp, f32, vp, i32, i32, vp, vp, vp,
                                                vp]),
     "egot2_grad_norm_groups": (C.c_int, [vp, sz, f32, vp, vp, vp, vp, vp, sz, vp]),
+    "egot2_sgd_step_fused": (C.c_int, [vp, vp, vp, sz, f32, vp, f32, f32, i32, f32, i32, vp, f32, vp, i32, vp, vp, vp, vp]),
     "egot2_gemm": (C.c_int, [i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, i32, i32, vp]),
     "egot2_gemm_last_impl": (C.c_char_p, []),
     "egot2_layernorm_fwd": (C.c_int, [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp]),

@@ -13,7 +13,8 @@
 // With a gradient guard (egot2_dp_desc.guard) step 2 is split at the global norm: dp_guard_reduce_kernel, then
 // dp_guard_adam_kernel (one more flag round trip, for the per-rank partial sums of squares).  With parameter groups
 // (egot2_dp_desc.groups) every quad takes its group's lr and weight decay, frozen quads are neither updated nor gathered
-// (only their gradient is cleared) and stay out of the guard's norm.
+// (only their gradient is cleared) and stay out of the guard's norm.  With egot2_dp_desc.sgd the update is torch.optim.SGD
+// (dp_reduce_sgd_kernel, or dp_guard_reduce_kernel + dp_guard_sgd_kernel) on the local momentum buffer; everything else is the same.
 // After the kernel every rank holds bit-identical parameters (each slice is computed once, by its owner), no rank reads a
 // peer's gradients any more (so the caller may clear its gradient arena), and nothing went through the host: the kernel sits in
 // the step's CUDA graph behind the backward pass.  The message is latency-bound for the translators (0.7-9 M parameters), which
@@ -55,6 +56,11 @@ struct DpArgs {
   egot2_grad_guard* guard;             // optional: global-norm clip / non-finite skip (two launches, see dp_guard_reduce_kernel)
   const egot2_param_groups* groups;    // optional: parameter groups, with the arena's block map
   const uint8_t* block_group;
+  // last, so that the Adam kernels keep their parameter offsets: torch.optim.SGD instead of Adam (m = the momentum buffer or
+  // NULL, v unused); first_step: the host step count is 1 (used without step_dev)
+  int sgd;
+  float momentum, dampening;
+  int nesterov, first_step;
 };
 
 __device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v) {
@@ -114,6 +120,33 @@ __device__ __forceinline__ void store_and_gather(const DpArgs& a, size_t q, cons
                                                  int zero_remote) {
   reinterpret_cast<float4*>(a.m)[q] = make_float4(mm[0], mm[1], mm[2], mm[3]);
   reinterpret_cast<float4*>(a.v)[q] = make_float4(vv[0], vv[1], vv[2], vv[3]);
+  const float4 wn = make_float4(w[0], w[1], w[2], w[3]);
+  __nv_bfloat162 s0 = __floats2bfloat162_rn(w[0], w[1]), s1 = __floats2bfloat162_rn(w[2], w[3]);
+  uint2 sh; sh.x = *reinterpret_cast<uint32_t*>(&s0); sh.y = *reinterpret_cast<uint32_t*>(&s1);
+  for (int p = 0; p < a.world; ++p) {
+    reinterpret_cast<float4*>(a.slab[p] + a.off_param)[q] = wn;
+    if (a.off_shadow != (size_t)-1) reinterpret_cast<uint2*>(a.slab[p] + a.off_shadow)[q] = sh;
+    if (zero_remote) reinterpret_cast<float4*>(a.slab[p] + a.off_grad)[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+}
+// the arithmetic of sgd_kernel (rowops.cu), element for element: bb is the momentum buffer (unused without momentum)
+__device__ __forceinline__ void sgd_quad(const DpArgs& a, float lr, float wd, bool first, const float* gg, float* w,
+                                         float* bb) {
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    float d = gg[k];
+    if (wd != 0.f) d += wd * w[k];
+    if (a.m) {
+      bb[k] = first ? d : a.momentum * bb[k] + (1.f - a.dampening) * d;
+      d = a.nesterov ? d + a.momentum * bb[k] : bb[k];
+    }
+    w[k] = w[k] - lr * d;
+  }
+}
+// SGD's store_and_gather: the local momentum buffer (if any), then the same all-gather of fp32 + bf16 shadow
+__device__ __forceinline__ void store_and_gather_sgd(const DpArgs& a, size_t q, const float* w, const float* bb,
+                                                     int zero_remote) {
+  if (a.m) reinterpret_cast<float4*>(a.m)[q] = make_float4(bb[0], bb[1], bb[2], bb[3]);
   const float4 wn = make_float4(w[0], w[1], w[2], w[3]);
   __nv_bfloat162 s0 = __floats2bfloat162_rn(w[0], w[1]), s1 = __floats2bfloat162_rn(w[2], w[3]);
   uint2 sh; sh.x = *reinterpret_cast<uint32_t*>(&s0); sh.y = *reinterpret_cast<uint32_t*>(&s1);
@@ -209,6 +242,64 @@ __global__ void __launch_bounds__(256) dp_reduce_adam_kernel(const DpArgs a) {
       float mm[4] = {m4[u].x, m4[u].y, m4[u].z, m4[u].w}, vv[4] = {v4[u].x, v4[u].y, v4[u].z, v4[u].w};
       adam_quad(a, lr_q, wd_q, bc1, bc2_sqrt, gg, w, mm, vv);
       store_and_gather(a, q, w, mm, vv, a.zero_remote);
+    }
+  }
+  finish_epoch(a, grid_ctr, done, epoch_w, e);
+}
+
+// dp_reduce_adam_kernel with the SGD update: the same flags, slice, rank-order sum and frozen quads
+__global__ void __launch_bounds__(256) dp_reduce_sgd_kernel(const DpArgs a) {
+  EGOT2_PDL_ENTER();
+  uint32_t* my_flags = reinterpret_cast<uint32_t*>(a.slab[a.rank] + a.off_flags) + a.channel * kChanWords;
+  uint32_t* arrive = my_flags;
+  uint32_t* done = my_flags + kMaxRanks;
+  uint32_t* epoch_w = my_flags + 2 * kMaxRanks;
+  uint32_t* grid_ctr = my_flags + 2 * kMaxRanks + 1;
+  const uint32_t e = *reinterpret_cast<volatile uint32_t*>(epoch_w) + 1;
+
+  if (blockIdx.x == 0 && threadIdx.x < a.world) {
+    st_release_sys(reinterpret_cast<uint32_t*>(a.slab[threadIdx.x] + a.off_flags) + a.channel * kChanWords + a.rank, e);
+  }
+  if (threadIdx.x < a.world) spin_until(arrive + threadIdx.x, e);
+  __syncthreads();
+
+  const bool first = a.step_dev ? *a.step_dev == 1 : a.first_step != 0;
+  const float lr = a.lr_dev ? *a.lr_dev : a.lr;
+  const float inv_world = 1.f / (float)a.world;
+  size_t q0, q1;
+  slice_quads(a, q0, q1);
+  constexpr int U = 2;
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t qb = q0 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; qb < q1; qb += stride * U) {
+    float4 g[U], w4[U], b4[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const size_t q = qb + u * stride;
+      g[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+      b4[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (q < q1) {
+        for (int p = 0; p < a.world; ++p) {      // rank order, as dp_reduce_adam_kernel
+          const float4 x = reinterpret_cast<const float4*>(a.slab[p] + a.off_grad)[q];
+          g[u].x += x.x; g[u].y += x.y; g[u].z += x.z; g[u].w += x.w;
+        }
+        w4[u] = reinterpret_cast<const float4*>(a.slab[a.rank] + a.off_param)[q];
+        if (a.m && !first) b4[u] = reinterpret_cast<float4*>(a.m)[q];
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const size_t q = qb + u * stride;
+      if (q >= q1) continue;
+      float lr_q, wd_q;
+      if (quad_hp(a, q, lr, lr_q, wd_q)) {       // frozen: parameters, shadow and buffer stay; the gradient is cleared
+        if (a.zero_remote) clear_grad_quad(a, q);
+        continue;
+      }
+      float gg[4] = {g[u].x * inv_world, g[u].y * inv_world, g[u].z * inv_world, g[u].w * inv_world};
+      float w[4] = {w4[u].x, w4[u].y, w4[u].z, w4[u].w};
+      float bb[4] = {b4[u].x, b4[u].y, b4[u].z, b4[u].w};
+      sgd_quad(a, lr_q, wd_q, first, gg, w, bb);
+      store_and_gather_sgd(a, q, w, bb, a.zero_remote);
     }
   }
   finish_epoch(a, grid_ctr, done, epoch_w, e);
@@ -342,6 +433,39 @@ __global__ void __launch_bounds__(256) dp_guard_adam_kernel(const DpArgs a) {
   finish_epoch(a, grid_ctr, done, epoch_w, e);
 }
 
+// Phase B of the guarded exchange with the SGD update (phase A, dp_guard_reduce_kernel, does not depend on the optimizer).
+// The step count phase A left is that of the applied steps, so a skipped first step leaves the buffer's initialisation to
+// the next applied one.
+__global__ void __launch_bounds__(256) dp_guard_sgd_kernel(const DpArgs a) {
+  EGOT2_PDL_ENTER();
+  uint32_t* my_flags = reinterpret_cast<uint32_t*>(a.slab[a.rank] + a.off_flags) + a.channel * kChanWords;
+  uint32_t* done = my_flags + kMaxRanks;
+  uint32_t* epoch_w = my_flags + 2 * kMaxRanks;
+  uint32_t* grid_ctr = my_flags + 2 * kMaxRanks + 1;
+  const uint32_t e = *reinterpret_cast<volatile uint32_t*>(epoch_w) + 1;
+  const bool skip = a.guard->skip != 0;
+  const float coef = a.guard->coef;
+  const bool first = a.step_dev ? *a.step_dev == 1 : a.first_step != 0;
+  const float lr = a.lr_dev ? *a.lr_dev : a.lr;
+  size_t q0, q1;
+  slice_quads(a, q0, q1);
+  float4* grad = reinterpret_cast<float4*>(a.slab[a.rank] + a.off_grad);
+  for (size_t q = q0 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; q < q1; q += (size_t)gridDim.x * blockDim.x) {
+    float lr_q, wd_q;
+    if (!skip && !quad_hp(a, q, lr, lr_q, wd_q)) {
+      const float4 g4 = grad[q], w4 = reinterpret_cast<const float4*>(a.slab[a.rank] + a.off_param)[q];
+      const float4 b4 = a.m && !first ? reinterpret_cast<float4*>(a.m)[q] : make_float4(0.f, 0.f, 0.f, 0.f);
+      float gg[4] = {g4.x * coef, g4.y * coef, g4.z * coef, g4.w * coef};
+      float w[4] = {w4.x, w4.y, w4.z, w4.w};
+      float bb[4] = {b4.x, b4.y, b4.z, b4.w};
+      sgd_quad(a, lr_q, wd_q, first, gg, w, bb);
+      store_and_gather_sgd(a, q, w, bb, 0);
+    }
+    if (a.zero_remote) grad[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  finish_epoch(a, grid_ctr, done, epoch_w, e);
+}
+
 }  // namespace
 }  // namespace egot2
 
@@ -386,7 +510,17 @@ extern "C" int egot2_dp_reduce_adam_range(const egot2_dp_desc* d, int64_t lo, in
 }
 static int dp_launch(const egot2_dp_desc* d, long long lo, long long hi, int channel, void* stream) {
   EGOT2_CHECK(d && d->world >= 1 && d->world <= kMaxRanks && d->rank >= 0 && d->rank < d->world, "dp_reduce_adam: world/rank");
-  EGOT2_CHECK(d->numel > 0 && d->numel % 4 == 0 && d->exp_avg && d->exp_avg_sq, "dp_reduce_adam: arena (numel %% 4 == 0) / moments");
+  EGOT2_CHECK(d->numel > 0 && d->numel % 4 == 0, "dp_reduce_adam: arena (numel %% 4 == 0)");
+  if (d->sgd) {
+    EGOT2_CHECK(d->momentum >= 0.f && isfinite(d->momentum) && isfinite(d->dampening) && !d->decoupled,
+                "dp_reduce_adam (sgd): momentum %g / dampening %g / decoupled %d", d->momentum, d->dampening, d->decoupled);
+    EGOT2_CHECK(!d->nesterov || (d->momentum > 0.f && d->dampening == 0.f),
+                "dp_reduce_adam (sgd): nesterov needs momentum > 0 and dampening 0");
+    EGOT2_CHECK((d->exp_avg == nullptr) == (d->momentum == 0.f),
+                "dp_reduce_adam (sgd): exp_avg (the momentum buffer) must be given exactly when momentum != 0");
+  } else {
+    EGOT2_CHECK(d->exp_avg && d->exp_avg_sq, "dp_reduce_adam: moments");
+  }
   EGOT2_CHECK(lo >= 0 && hi <= d->numel && lo <= hi && lo % 4 == 0 && hi % 4 == 0 && channel >= 0 && channel < kChannels,
               "dp_reduce_adam: range [%lld, %lld) / channel %d", lo, hi, channel);
   if (lo == hi) return 0;
@@ -414,6 +548,12 @@ static int dp_launch(const egot2_dp_desc* d, long long lo, long long hi, int cha
   EGOT2_CHECK(!d->groups == !d->block_group, "dp_reduce_adam: groups and block_group go together");
   a.groups = d->groups;
   a.block_group = d->block_group;
+  a.sgd = d->sgd ? 1 : 0;
+  a.momentum = d->momentum;
+  a.dampening = d->dampening;
+  a.nesterov = d->nesterov ? 1 : 0;
+  a.first_step = d->step == 1 ? 1 : 0;
+  EGOT2_CHECK(!a.sgd || d->step >= 1 || d->step_dev, "dp_reduce_adam (sgd): step must be >= 1");
   // a few CTAs per rank: the message is latency-bound, and the spinning CTAs must never crowd out other work
   const size_t per4 = ((size_t)(hi - lo) / 4 + d->world - 1) / d->world;
   // latency-bound for the small arenas (a few CTAs), bandwidth-bound for the large ones (two waves of resident CTAs)
@@ -424,13 +564,14 @@ static int dp_launch(const egot2_dp_desc* d, long long lo, long long hi, int cha
   if (grid < 1) grid = 1;
   a.zero_remote = d->zero_grads_remote ? 1 : 0;
   cudaStream_t st = (cudaStream_t)stream;
-  ProfScope prof(st, "dp_reduce_adam n%lld world%d ch%d", (long long)(hi - lo), d->world, channel);
+  ProfScope prof(st, a.sgd ? "dp_reduce_sgd n%lld world%d ch%d" : "dp_reduce_adam n%lld world%d ch%d", (long long)(hi - lo),
+                 d->world, channel);
   if (a.guard) {
     launch(dp_guard_reduce_kernel, dim3(grid), dim3(256), 0, st, a);
     EGOT2_LAUNCH_CHECK();
-    launch(dp_guard_adam_kernel, dim3(grid), dim3(256), 0, st, a);
+    launch(a.sgd ? dp_guard_sgd_kernel : dp_guard_adam_kernel, dim3(grid), dim3(256), 0, st, a);
   } else {
-    launch(dp_reduce_adam_kernel, dim3(grid), dim3(256), 0, st, a);
+    launch(a.sgd ? dp_reduce_sgd_kernel : dp_reduce_adam_kernel, dim3(grid), dim3(256), 0, st, a);
   }
   EGOT2_LAUNCH_CHECK();
   return 0;

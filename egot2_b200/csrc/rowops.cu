@@ -441,6 +441,65 @@ __global__ void adam_kernel(float* __restrict__ p, float* __restrict__ g, float*
   }
 }
 
+// torch.optim.SGD (coupled weight decay, momentum with dampening, Nesterov) in the same single pass as adam_kernel: guard,
+// device lr and step count, shadow write and gradient clear.  buf is NULL exactly when momentum == 0.  The momentum buffer
+// starts as the first applied step's gradient (torch: `buf is None` until a parameter's first optimizer.step()); that step
+// is the one whose count is 1 (*step_dev when given, else `first` from the host), so a skipped first step, whose count the
+// guard takes back, leaves the initialisation to the next applied one.  GROUPS as in adam_kernel.
+template <bool GROUPS>
+__global__ void sgd_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ buf, size_t n, float lr,
+                           float momentum, float dampening, int nesterov, float wd, int first, float gscale,
+                           bf16* __restrict__ shadow, int zero_grad, const int32_t* __restrict__ step_dev,
+                           const float* __restrict__ lr_dev, const egot2_grad_guard* __restrict__ guard,
+                           const egot2_param_groups* __restrict__ groups, const uint8_t* __restrict__ block_group) {
+  EGOT2_PDL_ENTER();
+  __shared__ float s_lr_mult[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1], s_wd[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1];
+  __shared__ int s_frozen[GROUPS ? EGOT2_MAX_PARAM_GROUPS : 1];
+  if (GROUPS) {
+    if (threadIdx.x < EGOT2_MAX_PARAM_GROUPS) {
+      s_lr_mult[threadIdx.x] = groups->lr_mult[threadIdx.x];
+      s_wd[threadIdx.x] = groups->weight_decay[threadIdx.x];
+      s_frozen[threadIdx.x] = groups->frozen[threadIdx.x];
+    }
+    __syncthreads();
+  }
+  if (guard) {               // egot2_grad_norm ran before: clip, or skip the update and only clear the gradient
+    if (guard->skip) {
+      if (zero_grad)
+        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) g[i] = 0.f;
+      return;
+    }
+    gscale *= guard->coef;
+  }
+  if (step_dev) first = *step_dev == 1;
+  if (lr_dev) lr = *lr_dev;
+  const float keep = 1.f - dampening;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    float lr_e = lr, wd_e = wd;
+    if (GROUPS) {
+      const int k = block_group[i >> 6];
+      if (s_frozen[k]) {                                 // requires_grad=False: only the gradient is cleared
+        if (zero_grad) g[i] = 0.f;
+        continue;
+      }
+      lr_e = lr * s_lr_mult[k];
+      wd_e = s_wd[k];
+    }
+    float d = g[i] * gscale;
+    const float w = p[i];
+    if (wd_e != 0.f) d += wd_e * w;
+    if (buf) {
+      const float b = first ? d : momentum * buf[i] + keep * d;
+      buf[i] = b;
+      d = nesterov ? d + momentum * b : b;
+    }
+    const float wn = w - lr_e * d;
+    p[i] = wn;
+    if (shadow) shadow[i] = __float2bfloat16_rn(wn);
+    if (zero_grad) g[i] = 0.f;
+  }
+}
+
 // lr_at of include/egot2.h, without the warm-up
 __device__ double lr_policy(const egot2_lr_sched& s, long long t) {
   if (s.kind == EGOT2_LR_COSINE) {
@@ -1188,6 +1247,27 @@ extern "C" int egot2_adam_step_fused_groups(float* param, float* grad, float* ex
               "adam: step_dev / groups / block_group is null");
   return adam_launch(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, 0.f, 1, grad_scale, shadow_bf16, zero_grad,
                      stream, step_dev, decoupled != 0, lr_dev, guard, groups, block_group);
+}
+
+extern "C" int egot2_sgd_step_fused(float* param, float* grad, float* momentum_buf, size_t n, float lr, const float* lr_dev,
+                                    float momentum, float dampening, int32_t nesterov, float weight_decay, int32_t step,
+                                    const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                                    const egot2_grad_guard* guard, const egot2_param_groups* groups,
+                                    const uint8_t* block_group, void* stream) {
+  EGOT2_CHECK(momentum >= 0.f && isfinite(momentum) && isfinite(dampening), "sgd: momentum %g / dampening %g", momentum,
+              dampening);
+  EGOT2_CHECK(!nesterov || (momentum > 0.f && dampening == 0.f), "sgd: nesterov needs momentum > 0 and dampening 0");
+  EGOT2_CHECK((momentum_buf == nullptr) == (momentum == 0.f), "sgd: momentum_buf must be given exactly when momentum != 0");
+  EGOT2_CHECK(step >= 1 || step_dev, "sgd: step must be >= 1");
+  EGOT2_CHECK(!guard || step_dev, "sgd: a guard needs step_dev (a skip takes the step back)");
+  EGOT2_CHECK(!groups || block_group || n == 0, "sgd: groups need block_group");
+  if (n == 0) return 0;
+  ProfScope prof((cudaStream_t)stream, groups ? "sgd_groups n%zu" : "sgd n%zu", n);
+  launch(groups ? sgd_kernel<true> : sgd_kernel<false>, dim3(ew_grid(n)), dim3(256), 0, (cudaStream_t)stream, param, grad,
+         momentum_buf, n, lr, momentum, dampening, nesterov ? 1 : 0, groups ? 0.f : weight_decay, step == 1 ? 1 : 0,
+         grad_scale, (bf16*)shadow_bf16, zero_grad, step_dev, lr_dev, guard, groups, block_group);
+  EGOT2_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" size_t egot2_grad_norm_workspace_bytes(void) { return kNormCtas * sizeof(double) + 16; }

@@ -867,6 +867,39 @@ class TranslatorEngine:
                float(grad_scale), _stream())
         self.arena.shadow_fresh = False
 
+    @_on_device
+    def sgd_step(self, state: Dict[str, torch.Tensor], step: int, lr: float, sgd, weight_decay: float = 0.0,
+                 grad_scale: float = 1.0, step_dev: Optional[torch.Tensor] = None, lr_dev: Optional[torch.Tensor] = None,
+                 guard: Optional[torch.Tensor] = None, groups: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+        """torch.optim.SGD (`sgd`: optim.SGD) over the whole arena in one egot2_sgd_step_fused launch, which also writes the
+        bf16 shadow (bf16 engines) and clears the gradient arena.  state["buf"] is the momentum buffer (only with momentum).
+        step / step_dev: the step count (host, or read on the device) whose value 1 initialises the buffer.  lr_dev, guard and
+        groups as in adam_step (lr_dev, guard and groups need step_dev); with a guard the norm launch runs first."""
+        if sgd.momentum != 0.0 and "buf" not in state:
+            state["buf"] = torch.zeros_like(self.arena.param)
+        if (lr_dev is not None or guard is not None or groups is not None) and step_dev is None:
+            raise L.Egot2Error("sgd_step: lr_dev, a gradient guard and parameter groups need step_dev")
+        shadow = None
+        if self.dtype == "bf16":
+            if self.arena.shadow is None:
+                self.arena.refresh_shadow()
+            shadow = self.arena.shadow.data_ptr()
+        desc, block_group = (None, None) if groups is None else (groups[0].data_ptr(), groups[1].data_ptr())
+        if guard is not None:
+            ws = self.grad_norm_workspace()
+            if groups is None:
+                L.call("egot2_grad_norm", self.arena.grad.data_ptr(), self.arena.numel, float(grad_scale),
+                       guard.data_ptr(), step_dev.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
+            else:
+                L.call("egot2_grad_norm_groups", self.arena.grad.data_ptr(), self.arena.numel, float(grad_scale),
+                       guard.data_ptr(), step_dev.data_ptr(), desc, block_group, ws.data_ptr(), ws.numel(), _stream())
+        L.call("egot2_sgd_step_fused", self.arena.param.data_ptr(), self.arena.grad.data_ptr(),
+               state["buf"].data_ptr() if sgd.momentum != 0.0 else None, self.arena.numel, float(lr),
+               None if lr_dev is None else lr_dev.data_ptr(), sgd.momentum, sgd.dampening, int(sgd.nesterov),
+               float(weight_decay), int(step), None if step_dev is None else step_dev.data_ptr(), float(grad_scale), shadow,
+               1, None if guard is None else guard.data_ptr(), desc, block_group, _stream())
+        self.arena.shadow_fresh = shadow is not None
+
     def grad_norm_workspace(self) -> torch.Tensor:
         """The egot2_grad_norm workspace of this engine: zero-filled once, and every launch leaves it so.  Trainers allocate it
         at construction, outside any CUDA-graph capture."""

@@ -13,6 +13,9 @@ with an optional linear warm-up.  Steps are optimizer steps; callers that think 
 `ParamGroup` is the fused trainers' form of torch.optim's param groups (per-group weight decay and lr multiplier, frozen
 parameters).  They are applied per element by the optimizer kernels, from a device-resident `egot2_param_groups` descriptor
 and a map of one group per 64-element block of the parameter arena (include/egot2.h); `resolve_param_groups` builds both.
+
+`SGD` selects torch.optim.SGD (momentum, dampening, Nesterov) instead of Adam / AdamW for a fused trainer
+(egot2_sgd_step_fused, egot2_dp_desc.sgd): SlowFast's construct_optimizer builds it beside Adam and AdamW (HOI/optimizers/).
 """
 from __future__ import annotations
 
@@ -165,3 +168,28 @@ def pack_param_groups(hp: Sequence[Tuple[float, float, bool]]) -> L.ParamGroups:
     for i, (lr_mult, wd, frozen) in enumerate(hp):
         d.lr_mult[i], d.weight_decay[i], d.frozen[i] = lr_mult, wd, int(frozen)
     return d
+
+
+@dataclass(frozen=True)
+class SGD:
+    """torch.optim.SGD(momentum, dampening, nesterov) for a fused trainer's `optimizer=`; lr and weight decay stay the trainer's
+    (lr / lr_schedule, weight_decay, param_groups).  The checks are torch's: momentum >= 0, dampening finite, Nesterov needs
+    momentum > 0 and dampening 0.  SlowFast's SGD default is SGD(momentum=0.9, nesterov=True) with weight_decay 1e-4."""
+    momentum: float = 0.0
+    dampening: float = 0.0
+    nesterov: bool = False
+
+    def __post_init__(self):
+        momentum, dampening = float(self.momentum), float(self.dampening)
+        if not (math.isfinite(momentum) and momentum >= 0.0):
+            raise ValueError(f"SGD: momentum must be finite and >= 0, got {momentum}")
+        if not math.isfinite(dampening):
+            raise ValueError(f"SGD: dampening must be finite, got {dampening}")
+        if self.nesterov and (momentum <= 0.0 or dampening != 0.0):
+            raise ValueError("SGD: Nesterov momentum requires a momentum and zero dampening")
+        object.__setattr__(self, "momentum", momentum)
+        object.__setattr__(self, "dampening", dampening)
+        object.__setattr__(self, "nesterov", bool(self.nesterov))
+
+    def to_dict(self) -> dict:
+        return dataclasses.asdict(self)

@@ -169,21 +169,30 @@ class PeerExchange:
 
     def step(self, state, step: int, hp, stream: int, step_dev: Optional[torch.Tensor] = None, decoupled: bool = False,
              lo: int = 0, hi: Optional[int] = None, channel: int = 0, lr_dev: Optional[torch.Tensor] = None,
-             guard: Optional[torch.Tensor] = None, groups: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+             guard: Optional[torch.Tensor] = None, groups: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, sgd=None):
         """The exchange + optimizer step of this rank for arena elements [lo, hi) (default: everything) on flag `channel`;
         afterwards that part of the gradient arena is cleared (stream order).  lr_dev: the learning rate is read from this
         device float when the kernel executes (optim.py), instead of hp["lr"].  guard: a device egot2_grad_guard - the
         update is clipped by the global norm of the rank-averaged gradient, or skipped on every rank when it is not finite
         (two launches); it must cover the whole arena.  groups: (device egot2_param_groups, block map of the whole arena), as
-        in engine.adam_step; hp["weight_decay"] is then unused."""
+        in engine.adam_step; hp["weight_decay"] is then unused.  sgd: an optim.SGD - torch.optim.SGD on this rank's slice
+        instead of Adam (engine.sgd_step's semantics; state["buf"] is the local momentum buffer, hp["betas"] / hp["eps"] and
+        `decoupled` are unused)."""
         import ctypes as C
         from . import _lib as L
         arena = self.engine.arena
-        if "m" not in state:
-            state["m"] = torch.zeros_like(arena.param)
-            state["v"] = torch.zeros_like(arena.param)
         d = self.desc
-        d.exp_avg, d.exp_avg_sq = state["m"].data_ptr(), state["v"].data_ptr()
+        if sgd is None:
+            if "m" not in state:
+                state["m"] = torch.zeros_like(arena.param)
+                state["v"] = torch.zeros_like(arena.param)
+            d.exp_avg, d.exp_avg_sq = state["m"].data_ptr(), state["v"].data_ptr()
+            d.sgd, d.momentum, d.dampening, d.nesterov = 0, 0.0, 0.0, 0
+        else:
+            if sgd.momentum != 0.0 and "buf" not in state:
+                state["buf"] = torch.zeros_like(arena.param)
+            d.exp_avg, d.exp_avg_sq = (state["buf"].data_ptr() if sgd.momentum != 0.0 else None), None
+            d.sgd, d.momentum, d.dampening, d.nesterov = 1, sgd.momentum, sgd.dampening, int(sgd.nesterov)
         d.lr, (d.beta1, d.beta2), d.eps, d.weight_decay = hp["lr"], hp["betas"], hp["eps"], hp["weight_decay"]
         d.step = int(step)
         d.step_dev = step_dev.data_ptr() if step_dev is not None else None

@@ -19,7 +19,7 @@ import torch
 
 from . import _lib as L
 from .engine import _ALIGN, Activations, TranslatorEngine
-from .optim import LRSchedule, ParamGroup, check_group_hp, pack_param_groups, resolve_param_groups
+from .optim import SGD, LRSchedule, ParamGroup, check_group_hp, pack_param_groups, resolve_param_groups
 from .parallel import allreduce_gradients
 from .specs import TranslatorSpec
 
@@ -87,13 +87,24 @@ class _OptimizerState:
     a group later would need a step count per group, since torch starts the bias correction of parameters that first get
     optimizer state late from step 1.
 
+    With `optimizer=optim.SGD(...)` every optimizer launch is torch.optim.SGD (engine.sgd_step, or the peer exchange with
+    egot2_dp_desc.sgd) instead of Adam / AdamW, with the same step count, lr, guard and groups arguments; opt_state then holds
+    one momentum buffer "buf" (none without momentum) and no Adam moments.  Momentum, dampening and Nesterov are launch
+    arguments captured in the graphs, so they are fixed at construction.
+
     Without any of them, nothing here adds a launch."""
 
     def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float,
                               max_grad_norm: Optional[float] = None,
-                              param_groups: Optional[Sequence[ParamGroup]] = None):
+                              param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None):
         if lr_schedule is not None and lr != default_lr:
             raise ValueError("pass either lr or lr_schedule, not both")
+        if optimizer is not None:
+            if not isinstance(optimizer, SGD):
+                raise ValueError(f"optimizer must be None (Adam / AdamW) or an optim.SGD, got {optimizer!r}")
+            if tuple(self.hp["betas"]) != (0.9, 0.999) or self.hp["eps"] != 1e-8:
+                raise ValueError("betas and eps belong to Adam: pass them or optimizer=SGD(...), not both")
+        self.sgd = optimizer
         self.max_grad_norm = None
         if max_grad_norm is not None:
             max_grad_norm = _check_max_grad_norm(max_grad_norm)
@@ -220,6 +231,31 @@ class _OptimizerState:
         self._step_dev_val = self.step_count
         return self._opt_args(self._step_dev)
 
+    def _alloc_opt_state(self):
+        """The optimizer state, before a capture: the Adam moments, or SGD's momentum buffer (none without momentum)."""
+        param = self.engine.arena.param
+        if self.sgd is None:
+            if "m" not in self.opt_state:
+                self.opt_state["m"] = torch.zeros_like(param)
+                self.opt_state["v"] = torch.zeros_like(param)
+        elif self.sgd.momentum != 0.0 and "buf" not in self.opt_state:
+            self.opt_state["buf"] = torch.zeros_like(param)
+
+    def _optimizer_launch(self, grad_scale: float = 1.0, decoupled: bool = False, fused: bool = True, **opt):
+        """The optimizer launch of every path without the peer exchange: Adam / AdamW (engine.adam_step), or SGD
+        (engine.sgd_step, always fused).  opt: the step_dev / lr_dev / guard / groups of _opt_args / _advance_eager."""
+        if self.sgd is None:
+            self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
+                                  self.hp["weight_decay"], grad_scale=grad_scale, fused=fused, decoupled=decoupled, **opt)
+        else:
+            self.engine.sgd_step(self.opt_state, self.step_count, self.hp["lr"], self.sgd, self.hp["weight_decay"],
+                                 grad_scale=grad_scale, **opt)
+
+    def _peer_step(self, stream: int, decoupled: bool = False, **kw):
+        """The peer exchange with this trainer's optimizer (`decoupled`: AdamW, unused with SGD)."""
+        self.peer.step(self.opt_state, self.step_count, self.hp, stream, decoupled=decoupled and self.sgd is None,
+                       sgd=self.sgd, **kw)
+
     def _opt_args(self, step_dev: torch.Tensor) -> dict:
         """step_dev / lr_dev (/ guard / groups) of an optimizer launch that reads the device step count."""
         opt = dict(step_dev=step_dev, lr_dev=None if self.lr_schedule is None else self._lr_dev)
@@ -233,13 +269,20 @@ class _OptimizerState:
         """What a run needs beyond the parameters (state_dict) to resume as if uninterrupted: the Adam moments keyed by
         parameter name, the step count (train_step calls), the schedule, the dropout epoch and, with a guard, max_grad_norm and
         the number of skipped steps (read from the device: this syncs), and with parameter groups every group's patterns,
-        frozen flag and current lr_mult / weight_decay (group 0 first).  Under the peer-memory exchange every rank holds the
-        moments of its own arena slice only: save and load per rank."""
+        frozen flag and current lr_mult / weight_decay (group 0 first).  With SGD, "momentum_buffer" (keyed by parameter
+        name; None without momentum) and "sgd" (its fields) take the place of the moments.  Under the peer-memory exchange
+        every rank holds the moments (or buffer) of its own arena slice only: save and load per rank."""
         arena = self.engine.arena
-        zeros = None if "m" in self.opt_state else torch.zeros_like(arena.param)
-        return {"step": self.step_count,
-                "exp_avg": arena.state_dict(self.opt_state.get("m", zeros)),
-                "exp_avg_sq": arena.state_dict(self.opt_state.get("v", zeros)),
+        if self.sgd is None:
+            zeros = None if "m" in self.opt_state else torch.zeros_like(arena.param)
+            opt = {"exp_avg": arena.state_dict(self.opt_state.get("m", zeros)),
+                   "exp_avg_sq": arena.state_dict(self.opt_state.get("v", zeros))}
+        else:
+            buf = None
+            if self.sgd.momentum != 0.0:
+                buf = arena.state_dict(self.opt_state["buf"] if "buf" in self.opt_state else torch.zeros_like(arena.param))
+            opt = {"momentum_buffer": buf, "sgd": self.sgd.to_dict()}
+        return {"step": self.step_count, **opt,
                 "lr_schedule": None if self.lr_schedule is None else self.lr_schedule.to_dict(),
                 "dropout_epoch": self._epoch,
                 "max_grad_norm": self.max_grad_norm,
@@ -252,6 +295,13 @@ class _OptimizerState:
                 for p, (lr_mult, wd, frozen) in zip(pats, self._group_hp)]
 
     def load_optimizer_state_dict(self, sd: dict):
+        saved_sgd = sd.get("sgd")
+        if (saved_sgd is None) != (self.sgd is None):
+            raise ValueError("optimizer state saved " + ("for Adam" if saved_sgd is None else "for SGD") +
+                             ": build the trainer with the same optimizer")
+        if saved_sgd is not None and SGD(**saved_sgd) != self.sgd:
+            raise ValueError(f"optimizer state saved for {SGD(**saved_sgd)}, this trainer runs {self.sgd}: momentum, "
+                             "dampening and nesterov are fixed at construction")
         if (sd["lr_schedule"] is None) != (self.lr_schedule is None):
             raise ValueError("optimizer state saved " + ("without" if sd["lr_schedule"] is None else "with") +
                              " an lr_schedule: build the trainer the same way")
@@ -266,7 +316,11 @@ class _OptimizerState:
                 raise ValueError("optimizer state saved with other parameter groups (patterns / frozen): build the trainer "
                                  "with the same param_groups")
         arena = self.engine.arena
-        for k, key in (("m", "exp_avg"), ("v", "exp_avg_sq")):
+        if self.sgd is None:
+            pairs = (("m", "exp_avg"), ("v", "exp_avg_sq"))
+        else:
+            pairs = (("buf", "momentum_buffer"),) if self.sgd.momentum != 0.0 else ()
+        for k, key in pairs:
             if k in self.opt_state:        # in place: captured graphs hold these buffers
                 self.opt_state[k].zero_()
             else:
@@ -341,15 +395,12 @@ class _PromptStepGraphs(_OptimizerState):
             arena.refresh_shadow()
         replay()
         if getattr(self, "peer", None) is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=decoupled,
-                           **self._advance_eager())
+            self._peer_step(_cur_stream(self.device), decoupled=decoupled, **self._advance_eager())
         else:
             scale = 1.0
             if self.world > 1:
                 scale = allreduce_gradients(arena.grad, self.pg)
-            self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                                  self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=decoupled,
-                                  **self._advance_eager())
+            self._optimizer_launch(scale, decoupled, **self._advance_eager())
         self._grad_clean = True
         if self.dropout_epoch:
             with _dev_guard(self.device):
@@ -369,7 +420,8 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
 
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
                  ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None,
-                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None):
+                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
+                 optimizer: Optional[SGD] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -399,7 +451,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -450,16 +502,16 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
             self.engine.arena.grad.zero_()
         total = self._fwd_bwd_all(feats, labels, self.step_count * 4)         # one arena, accumulated over the three
         if self.peer is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), **self._advance_eager())
+            self._peer_step(_cur_stream(self.device), **self._advance_eager())
             self._grad_clean = True
             return total
         scale = 1.0
         if self.world > 1:
             scale = allreduce_gradients(self.engine.arena.grad, self.pg)
         sched = self._advance_eager()      # a schedule needs the fused launch (the one that reads the device lr)
-        self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                              self.hp["weight_decay"], grad_scale=scale, fused=bool(sched), **sched)
-        self._grad_clean = bool(sched)     # the plain Adam launch leaves the gradients in place
+        fused = bool(sched) or self.sgd is not None
+        self._optimizer_launch(scale, fused=fused, **sched)
+        self._grad_clean = fused           # the plain Adam launch leaves the gradients in place
         return total
 
     train_stream_host = None     # bound below to TranslatorTrainer's implementation (same double-buffered host path)
@@ -477,7 +529,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
     def __init__(self, hidden=512, heads=8, layers=3, dropout=0.1, vocab=600, device="cuda:0", dtype: str = "bf16",
                  lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
                  lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None,
-                 param_groups: Optional[Sequence[ParamGroup]] = None):
+                 param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -509,7 +561,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups)
+        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups, optimizer)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -564,16 +616,14 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
             l = act.t["loss"][0] * ratio
             total = l if total is None else total + l
         if self.peer is not None:
-            self.peer.step(self.opt_state, self.step_count, self.hp, _cur_stream(self.device), decoupled=True,
-                           **self._advance_eager())
+            self._peer_step(_cur_stream(self.device), decoupled=True, **self._advance_eager())
             self._grad_clean = True
             return total
         scale = 1.0
         if self.world > 1:
             scale = allreduce_gradients(eng.arena.grad, self.pg)
-        # AdamW (decoupled decay) + bf16 shadow + gradient clear in one launch
-        eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=scale, fused=True, decoupled=True, **self._advance_eager())
+        # AdamW (decoupled decay; with SGD its coupled decay) + bf16 shadow + gradient clear in one launch
+        self._optimizer_launch(scale, True, **self._advance_eager())
         self._grad_clean = True
         return total
 
@@ -593,7 +643,8 @@ class TranslatorTrainer(_OptimizerState):
     def __init__(self, spec: TranslatorSpec, device, dtype: str = "bf16", lr: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
                  sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None,
-                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None):
+                 max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
+                 optimizer: Optional[SGD] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -646,7 +697,7 @@ class TranslatorTrainer(_OptimizerState):
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}
@@ -718,8 +769,7 @@ class TranslatorTrainer(_OptimizerState):
         g2.replay()
         dist.all_reduce(eng.arena.grad[:nb], group=self.pg)
         work.wait()
-        eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=1.0 / self.world, fused=True, **self._advance_eager())
+        self._optimizer_launch(1.0 / self.world, **self._advance_eager())
         self._grad_clean = True
         self._advance_epoch()
         return act.t["loss"][0]
@@ -745,9 +795,7 @@ class TranslatorTrainer(_OptimizerState):
             self.engine.arena.shadow_fresh = True
         self._grad_clean = True
         if self.graph_update:
-            if "m" not in self.opt_state:                 # optimizer state must exist before capture
-                self.opt_state["m"] = torch.zeros_like(self.engine.arena.param)
-                self.opt_state["v"] = torch.zeros_like(self.engine.arena.param)
+            self._alloc_opt_state()                       # optimizer state must exist before capture
             if self.world > 1 and self.peer is None:      # communicator warm-up outside the capture (grad arena is zero)
                 allreduce_gradients(self.engine.arena.grad, self.pg)
             if self.max_grad_norm is None:             # with a guard the device count is authoritative (skips)
@@ -784,15 +832,14 @@ class TranslatorTrainer(_OptimizerState):
                 nb, n = self.engine.arena.embed_numel, self.engine.arena.numel
                 self._peer_stream.wait_stream(cur)
                 with torch.cuda.stream(self._peer_stream):
-                    self.peer.step(self.opt_state, self.step_count, self.hp, self._peer_stream.cuda_stream,
-                                   step_dev=self._step_dev, lo=nb, hi=n, channel=0, lr_dev=self._graph_lr_dev(),
-                                   groups=self._groups)
+                    self._peer_step(self._peer_stream.cuda_stream, step_dev=self._step_dev, lo=nb, hi=n, channel=0,
+                                    lr_dev=self._graph_lr_dev(), groups=self._groups)
                 self.engine.backward(act, zero_grad=False, stage="embed")
                 self._bump_stream.wait_stream(cur)
                 with torch.cuda.stream(self._bump_stream):
                     self._advance_epoch()
-                self.peer.step(self.opt_state, self.step_count, self.hp, cur.cuda_stream, step_dev=self._step_dev,
-                               lo=0, hi=nb, channel=1, lr_dev=self._graph_lr_dev(), groups=self._groups)
+                self._peer_step(cur.cuda_stream, step_dev=self._step_dev, lo=0, hi=nb, channel=1,
+                                lr_dev=self._graph_lr_dev(), groups=self._groups)
                 cur.wait_stream(self._peer_stream)
                 cur.wait_stream(self._bump_stream)
                 self._grad_clean = True
@@ -832,15 +879,13 @@ class TranslatorTrainer(_OptimizerState):
         eng = self.engine
         opt = self._advance_eager() if step_dev is None else self._opt_args(step_dev)
         if self.peer is not None:                         # one kernel: reduce-scatter + Adam + all-gather over peer memory
-            self.peer.step(self.opt_state, self.step_count, self.hp, torch.cuda.current_stream(self.device).cuda_stream,
-                           **opt)
+            self._peer_step(torch.cuda.current_stream(self.device).cuda_stream, **opt)
             self._grad_clean = True
             return
         scale = 1.0
         if self.world > 1:
             scale = allreduce_gradients(eng.arena.grad, self.pg)            # ONE flat NCCL all-reduce (NVLink)
-        eng.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
-                      self.hp["weight_decay"], grad_scale=scale, fused=True, **opt)
+        self._optimizer_launch(scale, **opt)
         self._grad_clean = True
 
     # ------------------------------------------------------------------ host-buffer (end-to-end) step

@@ -41,6 +41,9 @@
  *                                egot2_dp_reduce_adam (egot2_dp_desc.guard)
  *   egot2_adam_step_fused_groups torch.optim param groups (per-group weight decay / lr multiplier, frozen parameters) over the
  *                                flat arena in the same one launch (SlowFast's construct_optimizer, HOI/optimizers/)
+ *   egot2_sgd_step_fused         torch.optim.SGD (momentum, dampening, Nesterov, coupled weight decay) over the flat arena,
+ *                                with the same device lr / guard / groups as the Adam entries and in egot2_dp_reduce_adam
+ *                                (egot2_dp_desc.sgd); SlowFast's construct_optimizer builds it (HOI/optimizers/)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -495,6 +498,26 @@ int egot2_grad_norm_groups(const float* grad, size_t n, float grad_scale, egot2_
                            const egot2_param_groups* groups, const uint8_t* block_group, void* workspace, size_t ws_bytes,
                            void* stream);
 
+/* torch.optim.SGD (maximize=False) over the flat arena in one launch.  For the elements of group k (without groups: one group
+ * with lr_mult 1 and `weight_decay`), with lr the step's learning rate (by value, or *lr_dev when lr_dev is not NULL) and
+ * g = grad * grad_scale (* guard->coef with a guard):
+ *   if wd != 0:    g += wd * param                                      (coupled weight decay)
+ *   if momentum:   buf = g on the first applied step, else momentum * buf + (1 - dampening) * g
+ *                  d = nesterov ? g + momentum * buf : buf
+ *   else           d = g
+ *   param -= lr * lr_mult[k] * d;  shadow = bf16(param) (shadow_bf16 not NULL);  grad = 0 (zero_grad)
+ * The first applied step is the one whose count is 1: *step_dev when step_dev is not NULL (read when the kernel executes,
+ * after a guard took back a skipped step), else `step`.  momentum_buf is NULL exactly when momentum == 0.  momentum >= 0,
+ * dampening finite, nesterov needs momentum > 0 and dampening == 0.  guard (needs step_dev): egot2_grad_norm[_groups] ran
+ * first; on a skip parameters, shadow and buffer stay and the gradient is only cleared.  groups (with block_group):
+ * egot2_adam_step_fused_groups' per-group lr_mult / weight_decay (`weight_decay` is then unused) / frozen, where a frozen
+ * group also keeps its buffer. */
+int egot2_sgd_step_fused(float* param, float* grad, float* momentum_buf, size_t n, float lr, const float* lr_dev,
+                         float momentum, float dampening, int32_t nesterov, float weight_decay,
+                         int32_t step, const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
+                         const egot2_grad_guard* guard, const egot2_param_groups* groups, const uint8_t* block_group,
+                         void* stream);
+
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
  * translator gradients after backward, then the optimizer on every rank.  Here that is ONE kernel (csrc/peer.cu): gradient
@@ -527,6 +550,11 @@ typedef struct {
   const egot2_param_groups* groups;   /* optional, with block_group: parameter groups (egot2_adam_step_fused_groups' semantics;
                                        * `weight_decay` above is then unused, and the guard's norm leaves frozen groups out) */
   const uint8_t* block_group;         /* the group of every 64-element block of the WHOLE arena (also for a [lo, hi) range) */
+  int32_t sgd;                        /* 1: torch.optim.SGD (egot2_sgd_step_fused's semantics) instead of Adam: exp_avg is the
+                                       * LOCAL momentum buffer, NULL exactly when momentum == 0; exp_avg_sq may be NULL; beta1,
+                                       * beta2 and eps are unused; decoupled must be 0.  0: Adam / AdamW as above */
+  float momentum, dampening;
+  int32_t nesterov;
 } egot2_dp_desc;
 int egot2_peer_alloc(size_t bytes, void** ptr);
 int egot2_peer_free(void* ptr);
