@@ -120,6 +120,26 @@ class ParamGroups(C.Structure):
                 ("frozen", i32 * MAX_PARAM_GROUPS)]
 
 
+STATS_BUCKETS = 1548
+
+
+class ParamStatsDesc(C.Structure):
+    _fields_ = [("every", i32), ("histograms", i32), ("n_params", i32), ("step", i32), ("grad_norm", f32)]
+
+
+class StatsParam(C.Structure):
+    _fields_ = [("offset", C.c_int64), ("numel", C.c_int64), ("has_grad", i32), ("first_unit", i32 * 2), ("n_units", i32 * 2)]
+
+
+class StatsUnit(C.Structure):
+    _fields_ = [("param", i32), ("array", i32), ("begin", C.c_int64), ("end", C.c_int64)]
+
+
+class ParamStat(C.Structure):
+    _fields_ = [("sum", C.c_double), ("sum_squares", C.c_double), ("min", f32), ("max", f32), ("norm", f32),
+                ("nonfinite", i32), ("num", C.c_int64)]
+
+
 class LrSched(C.Structure):
     _fields_ = [("kind", i32), ("n_milestones", i32), ("warmup_steps", C.c_int64), ("total_steps", C.c_int64),
                 ("base_lr", C.c_double), ("warmup_start_lr", C.c_double), ("end_lr", C.c_double),
@@ -221,6 +241,8 @@ SIGNATURES = {
                                                vp]),
     "egot2_grad_norm_groups": (C.c_int, [vp, sz, f32, vp, vp, vp, vp, vp, sz, vp]),
     "egot2_sgd_step_fused": (C.c_int, [vp, vp, vp, sz, f32, vp, f32, f32, i32, f32, i32, vp, f32, vp, i32, vp, vp, vp, vp]),
+    "egot2_param_stats_workspace_bytes": (sz, [i32, i32]),
+    "egot2_param_stats": (C.c_int, [vp, vp, f32, vp, vp, vp, i32, vp, i32, vp, vp, vp, vp, sz, vp]),
     "egot2_gemm": (C.c_int, [i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, i32, i32, vp]),
     "egot2_gemm_last_impl": (C.c_char_p, []),
     "egot2_layernorm_fwd": (C.c_int, [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp]),

@@ -15,6 +15,7 @@ from typing import Dict, List, Optional, Sequence
 import ctypes as C
 import os
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -22,6 +23,8 @@ from .engine import _ALIGN, Activations, TranslatorEngine
 from .optim import SGD, LRSchedule, ParamGroup, check_group_hp, pack_param_groups, resolve_param_groups
 from .parallel import allreduce_gradients
 from .specs import TranslatorSpec
+from . import stats as S
+from .stats import ParamStats
 
 
 def _cur_stream(device) -> int:
@@ -92,11 +95,18 @@ class _OptimizerState:
     one momentum buffer "buf" (none without momentum) and no Adam moments.  Momentum, dampening and Nesterov are launch
     arguments captured in the graphs, so they are fixed at construction.
 
+    With `param_stats` (stats.ParamStats) the trainer owns the egot2_param_stats descriptor, its tables, its outputs and its
+    workspace: every optimizer launch is preceded, after any gradient all-reduce and before the guard's norm, by one
+    egot2_param_stats launch on the same grad_scale, which on a due step records the statistics of the gradient the optimizer
+    receives and of the parameters before the update (grad_norms(), histograms()), and on any other step exits at once.  The
+    device step count is then authoritative on every path, as with a guard or groups, so the due test is the same everywhere.
+
     Without any of them, nothing here adds a launch."""
 
     def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float,
                               max_grad_norm: Optional[float] = None,
-                              param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None):
+                              param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None,
+                              param_stats: Optional[ParamStats] = None):
         if lr_schedule is not None and lr != default_lr:
             raise ValueError("pass either lr or lr_schedule, not both")
         if optimizer is not None:
@@ -128,6 +138,7 @@ class _OptimizerState:
             self.set_max_grad_norm(max_grad_norm)
         self.param_groups = None
         self._groups = None
+        bmap = None
         if param_groups is not None:
             param_groups = list(param_groups)
             arena = self.engine.arena
@@ -140,6 +151,98 @@ class _OptimizerState:
             self._groups = (torch.zeros(C.sizeof(L.ParamGroups), device=self.device, dtype=torch.uint8),
                             torch.from_numpy(bmap).to(self.device))
             self._write_param_groups()
+        self.param_stats = None
+        self._stats = None
+        if param_stats is not None:
+            self._init_param_stats(param_stats, bmap)
+
+    def _init_param_stats(self, ps: ParamStats, bmap):
+        if not isinstance(ps, ParamStats):
+            raise ValueError(f"param_stats must be None or a stats.ParamStats, got {ps!r}")
+        if getattr(self, "peer", None) is not None:
+            raise ValueError("param_stats is not supported with the peer-memory exchange, which never materialises the "
+                             "rank-mean gradient: set EGOT2_DP_FUSED=0 (the NCCL all-reduce path) for statistics on several "
+                             "GPUs")
+        arena = self.engine.arena
+        names = list(arena.shapes)
+        frozen = [False] * len(names) if bmap is None else \
+            [self._group_hp[int(bmap[arena.offsets[n] // _ALIGN])][2] for n in names]
+        params, units = S.plan_units(arena.shapes, arena.offsets, [not f for f in frozen])
+        dev = self.device
+
+        def upload(obj):
+            return torch.frombuffer(bytearray(bytes(obj)), dtype=torch.uint8).to(dev)
+        P = len(names)
+        out = torch.zeros(S.buffer_bytes(P, ps.histograms), device=dev, dtype=torch.uint8)
+        out[:C.sizeof(L.ParamStatsDesc)].copy_(torch.frombuffer(bytearray(S.pack_desc(ps, P)), dtype=torch.uint8))
+        edges = torch.from_numpy(S.default_edges()).to(dev) if ps.histograms else None
+        ws = torch.zeros(int(L.load().egot2_param_stats_workspace_bytes(P, len(units))), device=dev, dtype=torch.uint8)
+        self.param_stats = ps
+        self._stats = dict(names=names, has_grad=[not f for f in frozen], params=upload(params), units=upload(units),
+                           n_units=len(units), out=out, edges=edges, ws=ws)
+
+    def _stats_launch(self, grad_scale: float, step_dev: torch.Tensor):
+        """egot2_param_stats on the gradient arena and the parameters, right before an optimizer launch (current stream)."""
+        st, arena = self._stats, self.engine.arena
+        P = len(st["names"])
+        base = st["out"].data_ptr()
+        counts = None if st["edges"] is None else base + S.stats_offset() + 2 * P * C.sizeof(L.ParamStat)
+        with _dev_guard(self.device):
+            L.call("egot2_param_stats", arena.grad.data_ptr(), arena.param.data_ptr(), float(grad_scale), step_dev.data_ptr(),
+                   base, st["params"].data_ptr(), P, st["units"].data_ptr(), st["n_units"],
+                   None if st["edges"] is None else st["edges"].data_ptr(), base + S.stats_offset(), counts,
+                   st["ws"].data_ptr(), st["ws"].numel(), _cur_stream(self.device))
+
+    def _check_stats(self):
+        if self.param_stats is None:
+            raise ValueError("this trainer was built without param_stats; no statistics are taken")
+
+    @property
+    def param_stats_step(self) -> torch.Tensor:
+        """The optimizer step count t of the last step the statistics were taken on (0: none yet), as a 0-dim device int32
+        tensor: no sync."""
+        self._check_stats()
+        f = L.ParamStatsDesc.step
+        return self._stats["out"][f.offset:f.offset + 4].view(torch.int32)[0]
+
+    def grad_norms(self) -> Dict[str, torch.Tensor]:
+        """{name: L2 norm of that parameter's gradient, ..., "total": over every trainable parameter} of the last due step,
+        as 0-dim device fp32 views (no sync): Lightning's grad_norm(module, 2).  Frozen parameters have no entry."""
+        self._check_stats()
+        st = self._stats
+        rec = C.sizeof(L.ParamStat) // 4
+        off = S.stats_offset()
+        f = st["out"][off:off + 2 * len(st["names"]) * C.sizeof(L.ParamStat)].view(torch.float32)
+        norms = {n: f[p * rec + L.ParamStat.norm.offset // 4] for p, n in enumerate(st["names"]) if st["has_grad"][p]}
+        g = L.ParamStatsDesc.grad_norm
+        norms["total"] = st["out"][g.offset:g.offset + 4].view(torch.float32)[0]
+        return norms
+
+    def histograms(self):
+        """(t, [(tag, add_histogram_raw kwargs), ...]) of the last due step t (0 and [] before the first): "name" for the
+        weights before the update and "name.grad" for the gradient the optimizer received, of every parameter with a
+        gradient.  Syncs: one device-to-host copy of the statistics and their bucket counts."""
+        self._check_stats()
+        if not self.param_stats.histograms:
+            raise ValueError("this trainer was built with ParamStats(histograms=False): only grad_norms() is available")
+        st = self._stats
+        P = len(st["names"])
+        host = st["out"].cpu().numpy().tobytes()
+        desc, recs = S.read_stats(host, P)
+        if desc.step == 0:
+            return 0, []
+        c0 = S.stats_offset() + 2 * P * C.sizeof(L.ParamStat)
+        counts = np.frombuffer(host[c0:], dtype=np.int32).reshape(2, P, L.STATS_BUCKETS)
+        edges = S.default_edges()
+        out = []
+        for p, n in enumerate(st["names"]):
+            for a, tag in ((1, n), (0, n + ".grad")):
+                if a == 0 and not st["has_grad"][p]:
+                    continue
+                h = S.histogram_raw(recs[a * P + p], counts[a, p], edges)
+                if h is not None:
+                    out.append((tag, h))
+        return int(desc.step), out
 
     def _write_param_groups(self):
         host = torch.frombuffer(bytearray(bytes(pack_param_groups(self._group_hp))), dtype=torch.uint8)
@@ -217,10 +320,10 @@ class _OptimizerState:
                    stream)
 
     def _advance_eager(self) -> dict:
-        """Before an eager optimizer launch: with a schedule, a guard or parameter groups, advance the device step count (and
+        """Before an eager optimizer launch: with a schedule, a guard, parameter groups or statistics, advance the device step count (and
         lr) on the current stream and return the launch's step_dev / lr_dev / guard / groups arguments; without any, nothing
         ({})."""
-        if self.lr_schedule is None and self.max_grad_norm is None and self._groups is None:
+        if self.lr_schedule is None and self.max_grad_norm is None and self._groups is None and self._stats is None:
             return {}
         if self.max_grad_norm is None and self._step_dev_val != self.step_count - 1:
             self._step_dev.fill_(self.step_count - 1)      # with a guard the device count is authoritative (skips)
@@ -243,7 +346,10 @@ class _OptimizerState:
 
     def _optimizer_launch(self, grad_scale: float = 1.0, decoupled: bool = False, fused: bool = True, **opt):
         """The optimizer launch of every path without the peer exchange: Adam / AdamW (engine.adam_step), or SGD
-        (engine.sgd_step, always fused).  opt: the step_dev / lr_dev / guard / groups of _opt_args / _advance_eager."""
+        (engine.sgd_step, always fused).  opt: the step_dev / lr_dev / guard / groups of _opt_args / _advance_eager.  With
+        statistics, egot2_param_stats runs first, on the same gradient and grad_scale."""
+        if self._stats is not None:
+            self._stats_launch(grad_scale, opt["step_dev"])
         if self.sgd is None:
             self.engine.adam_step(self.opt_state, self.step_count, self.hp["lr"], self.hp["betas"], self.hp["eps"],
                                   self.hp["weight_decay"], grad_scale=grad_scale, fused=fused, decoupled=decoupled, **opt)
@@ -421,7 +527,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
                  ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None,
                  max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
-                 optimizer: Optional[SGD] = None):
+                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -451,7 +557,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -529,7 +635,8 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
     def __init__(self, hidden=512, heads=8, layers=3, dropout=0.1, vocab=600, device="cuda:0", dtype: str = "bf16",
                  lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
                  lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None,
-                 param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None):
+                 param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None,
+                 param_stats: Optional[ParamStats] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -561,7 +668,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups, optimizer)
+        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups, optimizer, param_stats)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -644,7 +751,7 @@ class TranslatorTrainer(_OptimizerState):
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
                  sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None,
                  max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
-                 optimizer: Optional[SGD] = None):
+                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -697,7 +804,7 @@ class TranslatorTrainer(_OptimizerState):
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}

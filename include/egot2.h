@@ -44,6 +44,9 @@
  *   egot2_sgd_step_fused         torch.optim.SGD (momentum, dampening, Nesterov, coupled weight decay) over the flat arena,
  *                                with the same device lr / guard / groups as the Adam entries and in egot2_dp_reduce_adam
  *                                (egot2_dp_desc.sgd); SlowFast's construct_optimizer builds it (HOI/optimizers/)
+ *   egot2_param_stats            the add_histogram(name, weight) / add_histogram(name.grad, weight.grad) of the HOI LTA task's
+ *                                gradient logging every LOG_GRADIENT_PERIOD steps (HOI/tasks/lta/video_task.py:112-125)
+ *                                and Lightning's grad_norm, per parameter, on the device
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -517,6 +520,60 @@ int egot2_sgd_step_fused(float* param, float* grad, float* momentum_buf, size_t 
                          int32_t step, const int32_t* step_dev, float grad_scale, void* shadow_bf16, int32_t zero_grad,
                          const egot2_grad_guard* guard, const egot2_param_groups* groups, const uint8_t* block_group,
                          void* stream);
+
+/* Per-parameter statistics of the gradient and of the weights (the histograms and gradient norms a training loop logs every
+ * LOG_GRADIENT_PERIOD steps), on the device.  Array 0 is the gradient the optimizer applies, fp32(grad[i] * grad_scale);
+ * array 1 is the fp32 parameters.  A step t (*step_dev, read when the kernel executes) is due when (t - 1) % every == 0; on
+ * any other step every CTA returns at once and no output changes.  A DEVICE-resident descriptor: every, histograms and
+ * n_params are inputs, grad_norm and step are written on a due step, step last. */
+#define EGOT2_STATS_BUCKETS 1548      /* TensorBoard's default histogram: 1549 edges, see egot2_param_stats */
+typedef struct {
+  int32_t every;                      /* > 0 */
+  int32_t histograms;                 /* 1: bucket counts as well (needs edges and counts) */
+  int32_t n_params;                   /* P */
+  int32_t step;                       /* out: t of the last due step, 0 before the first */
+  float grad_norm;                    /* out: L2 norm of array 0 over the parameters with has_grad (NaN / inf as torch) */
+} egot2_param_stats_desc;
+/* One parameter of the arena: elements [offset, offset + numel).  has_grad = 0 (a frozen parameter): no gradient statistics,
+ * no units in array 0, and no share in grad_norm.  first_unit[a] / n_units[a]: its units of array a, consecutive. */
+typedef struct {
+  int64_t offset;
+  int64_t numel;
+  int32_t has_grad;
+  int32_t first_unit[2];
+  int32_t n_units[2];
+} egot2_stats_param;
+/* One work unit: arena elements [begin, end) of parameter `param` in array `array` (0 gradient, 1 weights).  Units are
+ * enumerated on the host, ordered by (array, param, begin); a unit never covers two parameters. */
+typedef struct {
+  int32_t param;
+  int32_t array;
+  int64_t begin, end;
+} egot2_stats_unit;
+/* The statistics of one (array, parameter); stats[a * P + p].  min / max / sum / sum_squares cover the finite elements (sums
+ * in fp64, added in a fixed order: bit-reproducible); nonfinite counts NaN and +-inf; norm = sqrt(sum_squares) as fp32, or NaN
+ * when a NaN is present, else +inf when an inf is; no finite element: min = +inf, max = -inf.  num = numel. */
+typedef struct {
+  double sum;
+  double sum_squares;
+  float min, max;
+  float norm;
+  int32_t nonfinite;
+  int64_t num;
+} egot2_param_stat;
+/* Bytes of the egot2_param_stats workspace for P parameters and n_units units.  Zero-fill it once (256-byte aligned); every
+ * call leaves it that way again, so the call can sit in a CUDA graph. */
+size_t egot2_param_stats_workspace_bytes(int32_t n_params, int32_t n_units);
+/* One launch of a grid fixed at launch: every unit's fp64 partial sums (fixed order), exact min / max / counts through integer
+ * atomics, the unit partials of a parameter added in unit order by the CTA that finishes its last unit.  With histograms,
+ * counts[a * P + p][b] = the number of finite values x with edges[b] <= (double)x < edges[b + 1] (the last bucket closed on
+ * the right; np.histogram's rule; -0.0 counts as 0).  edges: the 1549 doubles of TensorBoard's default bins
+ * (SummaryWriter.default_bins: v = 1e-12, times 1.1 while v < 1e20, mirrored, with 0).  edges and counts are both NULL
+ * without histograms.  No host sync; graph-capturable. */
+int egot2_param_stats(const float* grad, const float* param, float grad_scale, const int32_t* step_dev,
+                      egot2_param_stats_desc* desc, const egot2_stats_param* params, int32_t n_params,
+                      const egot2_stats_unit* units, int32_t n_units, const double* edges, egot2_param_stat* stats,
+                      int32_t* counts, void* workspace, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
