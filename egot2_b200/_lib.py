@@ -14,6 +14,7 @@ F32, BF16 = 0, 1
 LOSS_NONE, LOSS_CE, LOSS_BCE_SIGMOID, LOSS_CE_GROUPS = 0, 1, 2, 3
 LR_CONSTANT, LR_COSINE, LR_STEPS = 0, 1, 2
 LR_MAX_MILESTONES = 8
+AVG_EMA, AVG_SWA = 0, 1
 
 # EGOT2_LIB: an alternative build of the same library (instrumented / experimental variants for tools/); never a fallback
 _LIB_PATH = os.environ.get("EGOT2_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libegot2.so")
@@ -243,6 +244,7 @@ SIGNATURES = {
     "egot2_sgd_step_fused": (C.c_int, [vp, vp, vp, sz, f32, vp, f32, f32, i32, f32, i32, vp, f32, vp, i32, vp, vp, vp, vp]),
     "egot2_param_stats_workspace_bytes": (sz, [i32, i32]),
     "egot2_param_stats": (C.c_int, [vp, vp, f32, vp, vp, vp, i32, vp, i32, vp, vp, vp, vp, sz, vp]),
+    "egot2_weight_avg_update": (C.c_int, [vp, vp, sz, i32, f32, i32, i32, vp, vp, vp]),
     "egot2_gemm": (C.c_int, [i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, i32, i32, vp]),
     "egot2_gemm_last_impl": (C.c_char_p, []),
     "egot2_layernorm_fwd": (C.c_int, [i32, i32, i32, vp, vp, vp, f32, vp, vp, vp]),

@@ -16,6 +16,9 @@ and a map of one group per 64-element block of the parameter arena (include/egot
 
 `SGD` selects torch.optim.SGD (momentum, dampening, Nesterov) instead of Adam / AdamW for a fused trainer
 (egot2_sgd_step_fused, egot2_dp_desc.sgd): SlowFast's construct_optimizer builds it beside Adam and AdamW (HOI/optimizers/).
+
+`WeightAverage` selects an averaged copy of the weights (torch.optim.swa_utils.AveragedModel: EMA or SWA), kept by one
+egot2_weight_avg_update launch after every optimizer launch.
 """
 from __future__ import annotations
 
@@ -193,3 +196,57 @@ class SGD:
 
     def to_dict(self) -> dict:
         return dataclasses.asdict(self)
+
+
+_INT32_MAX = 2 ** 31 - 1
+
+
+@dataclass(frozen=True)
+class WeightAverage:
+    """An averaged copy of a fused trainer's parameters (`weight_average=`), updated on the device by egot2_weight_avg_update
+    after every due step: torch.optim.swa_utils.AveragedModel fed with the trainer's parameters.  Step t (the optimizer's
+    applied-step count, 1-based) is due when t >= start and (t - start) % every == 0; the first due step copies the
+    parameters, every later one lerps towards them.  Build with the constructors below."""
+    kind: int
+    decay: float = 0.0
+    every: int = 1
+    start: int = 1
+
+    @classmethod
+    def ema(cls, decay: float = 0.999, every: int = 1, start: int = 1) -> "WeightAverage":
+        """AveragedModel(multi_avg_fn=get_ema_multi_avg_fn(decay)): avg = lerp(avg, param, 1 - decay)."""
+        return cls(L.AVG_EMA, decay, every, start)
+
+    @classmethod
+    def swa(cls, every: int = 1, start: int = 1) -> "WeightAverage":
+        """AveragedModel() with its default average: the equal-weight running mean of the parameters on the due steps."""
+        return cls(L.AVG_SWA, 0.0, every, start)
+
+    def __post_init__(self):
+        if self.kind not in (L.AVG_EMA, L.AVG_SWA):
+            raise ValueError(f"WeightAverage: unknown kind {self.kind!r}")
+        try:
+            decay = float(self.decay)
+        except (TypeError, ValueError):
+            decay = math.nan
+        if not (math.isfinite(decay) and 0.0 <= decay <= 1.0):
+            raise ValueError(f"WeightAverage: decay must be finite and in [0, 1], got {self.decay!r}")
+        for name in ("every", "start"):
+            v = getattr(self, name)
+            if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 0 < int(v) <= _INT32_MAX:
+                raise ValueError(f"WeightAverage: {name} must be a positive int that fits in int32, got {v!r}")
+            object.__setattr__(self, name, int(v))
+        object.__setattr__(self, "decay", decay)
+
+    @property
+    def ema_weight(self) -> float:
+        """The lerp weight of an EMA update, float(1 - decay) with the subtraction in double as torch does it (0 for SWA,
+        whose weight the kernel computes from the update count)."""
+        return 1.0 - self.decay if self.kind == L.AVG_EMA else 0.0
+
+    def to_dict(self) -> dict:
+        return dataclasses.asdict(self)
+
+    @classmethod
+    def from_dict(cls, d: dict) -> "WeightAverage":
+        return cls(**{k: d[k] for k in ("kind", "decay", "every", "start")})

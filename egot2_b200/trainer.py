@@ -12,6 +12,7 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Sequence
 
+import contextlib
 import ctypes as C
 import os
 
@@ -20,7 +21,8 @@ import torch
 
 from . import _lib as L
 from .engine import _ALIGN, Activations, TranslatorEngine
-from .optim import SGD, LRSchedule, ParamGroup, check_group_hp, pack_param_groups, resolve_param_groups
+from .optim import (SGD, LRSchedule, ParamGroup, WeightAverage, check_group_hp, pack_param_groups,
+                    resolve_param_groups)
 from .parallel import allreduce_gradients
 from .specs import TranslatorSpec
 from . import stats as S
@@ -101,12 +103,19 @@ class _OptimizerState:
     receives and of the parameters before the update (grad_norms(), histograms()), and on any other step exits at once.  The
     device step count is then authoritative on every path, as with a guard or groups, so the due test is the same everywhere.
 
+    With `weight_average` (optim.WeightAverage) the trainer owns one more fp32 buffer of the arena's layout, the averaged
+    weights (torch.optim.swa_utils.AveragedModel over the trainer's parameters), and every step ends with one
+    egot2_weight_avg_update launch after its last optimizer launch (or peer exchange), on the trainer's device step count and
+    guard: a due step updates the average, a step the guard skipped leaves it alone.  The device step count is then
+    authoritative on every path.  Kind, decay, every and start are launch arguments captured in the graphs, so they are fixed
+    at construction.  averaged_state_dict() reads the average, averaged_weights() evaluates on it.
+
     Without any of them, nothing here adds a launch."""
 
     def _init_optimizer_state(self, lr_schedule: Optional[LRSchedule], lr: float, default_lr: float,
                               max_grad_norm: Optional[float] = None,
                               param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None,
-                              param_stats: Optional[ParamStats] = None):
+                              param_stats: Optional[ParamStats] = None, weight_average: Optional[WeightAverage] = None):
         if lr_schedule is not None and lr != default_lr:
             raise ValueError("pass either lr or lr_schedule, not both")
         if optimizer is not None:
@@ -155,6 +164,11 @@ class _OptimizerState:
         self._stats = None
         if param_stats is not None:
             self._init_param_stats(param_stats, bmap)
+        if weight_average is not None and not isinstance(weight_average, WeightAverage):
+            raise ValueError(f"weight_average must be None or an optim.WeightAverage, got {weight_average!r}")
+        self.weight_average = weight_average
+        self._avg = None if weight_average is None else torch.zeros_like(self.engine.arena.param)
+        self._in_averaged = False
 
     def _init_param_stats(self, ps: ParamStats, bmap):
         if not isinstance(ps, ParamStats):
@@ -244,6 +258,68 @@ class _OptimizerState:
                     out.append((tag, h))
         return int(desc.step), out
 
+    def _avg_launch(self, stream: int):
+        """egot2_weight_avg_update after the last optimizer launch of a step, on `stream`."""
+        wa, arena = self.weight_average, self.engine.arena
+        guard = None if self.max_grad_norm is None else self._guard_dev.data_ptr()
+        with _dev_guard(self.device):
+            L.call("egot2_weight_avg_update", arena.param.data_ptr(), self._avg.data_ptr(), arena.numel, wa.kind,
+                   wa.ema_weight, wa.every, wa.start, self._step_dev.data_ptr(), guard, stream)
+
+    def _check_weight_average(self):
+        if self.weight_average is None:
+            raise ValueError("this trainer was built without weight_average; it keeps no averaged weights")
+
+    def _check_training_weights(self):
+        if self._in_averaged:
+            raise ValueError("train_step inside averaged_weights(): the arena holds the averaged weights; leave the block "
+                             "first")
+
+    def _averaged_updates(self) -> int:
+        """The number of updates the average has taken (AveragedModel.n_averaged), from the device step count: syncs."""
+        self._check_weight_average()
+        wa, t = self.weight_average, int(self._step_dev[0])
+        return 0 if t < wa.start else (t - wa.start) // wa.every + 1
+
+    def _check_averaged(self):
+        if self._averaged_updates() == 0:
+            raise ValueError(f"no step has updated the average yet (the first update is at step {self.weight_average.start})")
+
+    def averaged_state_dict(self) -> Dict[str, torch.Tensor]:
+        """{reference state_dict name: fp32 tensor}: a copy of the averaged weights, which loads into the drop-in nn.Modules
+        as they are.  Reads the device step count (one sync) and raises ValueError before the first update."""
+        self._check_averaged()
+        return self.engine.arena.state_dict(self._avg)
+
+    @contextlib.contextmanager
+    def averaged_weights(self):
+        """Inside the block the arena holds the averaged weights and their bf16 shadow, so infer(), state_dict() and any
+        forward through the engine see them; train_step raises ValueError.  On exit the training parameters and shadow are
+        back bit for bit and training goes on as if the block never ran.  No graph is re-captured: the graphs read the arena
+        in place.  Raises ValueError before the first update (one sync).  Under data parallelism the peer exchange writes
+        into every rank's arena, so no rank may train while any rank is inside the block."""
+        self._check_averaged()
+        if self._in_averaged:
+            raise ValueError("averaged_weights() is already active")
+        arena = self.engine.arena
+        param = arena.param.clone()
+        shadow = None if arena.shadow is None else arena.shadow.clone()
+        fresh = arena.shadow_fresh
+        arena.param.copy_(self._avg)
+        arena.shadow_fresh = False
+        if self.engine.dtype == "bf16":
+            arena.refresh_shadow()
+            arena.shadow_fresh = True
+        self._in_averaged = True
+        try:
+            yield
+        finally:
+            arena.param.copy_(param)
+            if shadow is not None:
+                arena.shadow.copy_(shadow)
+            arena.shadow_fresh = fresh
+            self._in_averaged = False
+
     def _write_param_groups(self):
         host = torch.frombuffer(bytearray(bytes(pack_param_groups(self._group_hp))), dtype=torch.uint8)
         self._groups[0].copy_(host, non_blocking=True)          # pageable source: staged before copy_ returns
@@ -320,10 +396,11 @@ class _OptimizerState:
                    stream)
 
     def _advance_eager(self) -> dict:
-        """Before an eager optimizer launch: with a schedule, a guard, parameter groups or statistics, advance the device step count (and
-        lr) on the current stream and return the launch's step_dev / lr_dev / guard / groups arguments; without any, nothing
-        ({})."""
-        if self.lr_schedule is None and self.max_grad_norm is None and self._groups is None and self._stats is None:
+        """Before an eager optimizer launch: with a schedule, a guard, parameter groups, statistics or a weight average, advance
+        the device step count (and lr) on the current stream and return the launch's step_dev / lr_dev / guard / groups
+        arguments; without any, nothing ({})."""
+        if self.lr_schedule is None and self.max_grad_norm is None and self._groups is None and self._stats is None \
+                and self._avg is None:
             return {}
         if self.max_grad_norm is None and self._step_dev_val != self.step_count - 1:
             self._step_dev.fill_(self.step_count - 1)      # with a guard the device count is authoritative (skips)
@@ -347,7 +424,8 @@ class _OptimizerState:
     def _optimizer_launch(self, grad_scale: float = 1.0, decoupled: bool = False, fused: bool = True, **opt):
         """The optimizer launch of every path without the peer exchange: Adam / AdamW (engine.adam_step), or SGD
         (engine.sgd_step, always fused).  opt: the step_dev / lr_dev / guard / groups of _opt_args / _advance_eager.  With
-        statistics, egot2_param_stats runs first, on the same gradient and grad_scale."""
+        statistics, egot2_param_stats runs first, on the same gradient and grad_scale; with a weight average,
+        egot2_weight_avg_update runs last."""
         if self._stats is not None:
             self._stats_launch(grad_scale, opt["step_dev"])
         if self.sgd is None:
@@ -356,11 +434,18 @@ class _OptimizerState:
         else:
             self.engine.sgd_step(self.opt_state, self.step_count, self.hp["lr"], self.sgd, self.hp["weight_decay"],
                                  grad_scale=grad_scale, **opt)
+        if self._avg is not None:
+            self._avg_launch(_cur_stream(self.device))
 
-    def _peer_step(self, stream: int, decoupled: bool = False, **kw):
-        """The peer exchange with this trainer's optimizer (`decoupled`: AdamW, unused with SGD)."""
+    def _peer_step(self, stream: int, decoupled: bool = False, average: bool = True, **kw):
+        """The peer exchange with this trainer's optimizer (`decoupled`: AdamW, unused with SGD), followed on the same stream
+        by the weight-average update when there is one and `average` (every rank holds the all-gathered parameters, so every
+        rank computes the same average).  average=False: one piece of a split exchange, whose caller updates the average
+        once both pieces are joined."""
         self.peer.step(self.opt_state, self.step_count, self.hp, stream, decoupled=decoupled and self.sgd is None,
                        sgd=self.sgd, **kw)
+        if average and self._avg is not None:
+            self._avg_launch(stream)
 
     def _opt_args(self, step_dev: torch.Tensor) -> dict:
         """step_dev / lr_dev (/ guard / groups) of an optimizer launch that reads the device step count."""
@@ -376,7 +461,8 @@ class _OptimizerState:
         parameter name, the step count (train_step calls), the schedule, the dropout epoch and, with a guard, max_grad_norm and
         the number of skipped steps (read from the device: this syncs), and with parameter groups every group's patterns,
         frozen flag and current lr_mult / weight_decay (group 0 first).  With SGD, "momentum_buffer" (keyed by parameter
-        name; None without momentum) and "sgd" (its fields) take the place of the moments.  Under the peer-memory exchange
+        name; None without momentum) and "sgd" (its fields) take the place of the moments.  "weight_average" is None, or the
+        WeightAverage fields and "average", the averaged weights keyed by parameter name.  Under the peer-memory exchange
         every rank holds the moments (or buffer) of its own arena slice only: save and load per rank."""
         arena = self.engine.arena
         if self.sgd is None:
@@ -393,7 +479,9 @@ class _OptimizerState:
                 "dropout_epoch": self._epoch,
                 "max_grad_norm": self.max_grad_norm,
                 "skipped_steps": 0 if self.max_grad_norm is None else int(self.skipped_steps),
-                "param_groups": None if self.param_groups is None else self._groups_state()}
+                "param_groups": None if self.param_groups is None else self._groups_state(),
+                "weight_average": None if self._avg is None else {**self.weight_average.to_dict(),
+                                                                  "average": arena.state_dict(self._avg)}}
 
     def _groups_state(self) -> List[dict]:
         pats = [None] + [list(g.patterns) for g in self.param_groups]
@@ -421,6 +509,13 @@ class _OptimizerState:
             if membership(saved_groups) != membership(None if self.param_groups is None else self._groups_state()):
                 raise ValueError("optimizer state saved with other parameter groups (patterns / frozen): build the trainer "
                                  "with the same param_groups")
+        saved_avg = sd.get("weight_average")
+        if (saved_avg is None) != (self.weight_average is None):
+            raise ValueError("optimizer state saved " + ("without" if saved_avg is None else "with") +
+                             " a weight_average: build the trainer the same way")
+        if saved_avg is not None and WeightAverage.from_dict(saved_avg) != self.weight_average:
+            raise ValueError(f"optimizer state saved for {WeightAverage.from_dict(saved_avg)}, this trainer keeps "
+                             f"{self.weight_average}: kind, decay, every and start are fixed at construction")
         arena = self.engine.arena
         if self.sgd is None:
             pairs = (("m", "exp_avg"), ("v", "exp_avg_sq"))
@@ -432,6 +527,9 @@ class _OptimizerState:
             else:
                 self.opt_state[k] = torch.zeros_like(arena.param)
             arena.load_state_dict(sd[key], base=self.opt_state[k])
+        if saved_avg is not None:          # in place: captured graphs hold the buffer
+            self._avg.zero_()
+            arena.load_state_dict(saved_avg["average"], base=self._avg)
         self.step_count = int(sd["step"])
         skipped = int(sd.get("skipped_steps", 0))
         self._step_dev.fill_(self.step_count - skipped)     # the device count counts applied steps
@@ -527,7 +625,8 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
     def __init__(self, hidden=256, heads=4, layers=3, dropout=0.1, device="cuda:0", dtype: str = "bf16", lr: float = 5e-4,
                  ratios=(1.0, 1.0, 1.0), process_group=None, lr_schedule: Optional[LRSchedule] = None,
                  max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
-                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None):
+                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None,
+                 weight_average: Optional[WeightAverage] = None):
         from .hhi import PositionalEncoding
         from .specs import hhi_g_spec
         self.device = torch.device(device)
@@ -557,7 +656,8 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats,
+                                   weight_average)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -601,6 +701,7 @@ class PromptTranslatorTrainer(_PromptStepGraphs):
         return total
 
     def train_step(self, feats: Sequence[torch.Tensor], labels: torch.Tensor, graph_key: Optional[int] = None):
+        self._check_training_weights()
         self.step_count += 1
         if self.use_graphs and graph_key is not None:
             return self._graph_step(lambda: self._fwd_bwd_all(feats, labels, 4 * (abs(graph_key) + 1)), graph_key, False)
@@ -636,7 +737,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
                  lr: float = 1e-4, weight_decay: float = 1e-4, ratios=(1.0, 1.0, 1.0), n_tasks: int = 3, process_group=None,
                  lr_schedule: Optional[LRSchedule] = None, max_grad_norm: Optional[float] = None,
                  param_groups: Optional[Sequence[ParamGroup]] = None, optimizer: Optional[SGD] = None,
-                 param_stats: Optional[ParamStats] = None):
+                 param_stats: Optional[ParamStats] = None, weight_average: Optional[WeightAverage] = None):
         from .hhi import PositionalEncoding
         from .specs import hoi_g_spec
         self.device = torch.device(device)
@@ -668,7 +769,8 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
         self._h2d: Dict[int, List[torch.Tensor]] = {}
         self.copy_stream = None if self.device.type != "cuda" else torch.cuda.Stream(device=self.device)
         self.loss_kind, self.class_weight = L.LOSS_CE, None
-        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups, optimizer, param_stats)
+        self._init_optimizer_state(lr_schedule, lr, 1e-4, max_grad_norm, param_groups, optimizer, param_stats,
+                                   weight_average)
 
     def load_state_dict(self, sd):
         self.engine.arena.load_state_dict(sd)
@@ -706,6 +808,7 @@ class HoiPromptTranslatorTrainer(_PromptStepGraphs):
 
     def train_step(self, feats: Sequence[torch.Tensor], labels: torch.Tensor, graph_key: Optional[int] = None):
         assert len(feats) == 12, "three batches x (pnr, oscc, slow, fast)"
+        self._check_training_weights()
         self.step_count += 1
         if self.use_graphs and graph_key is not None:
             return self._graph_step(lambda: self._fwd_bwd_all(feats, labels, 4 * (abs(graph_key) + 1)), graph_key, True)
@@ -751,7 +854,8 @@ class TranslatorTrainer(_OptimizerState):
                  eps: float = 1e-8, weight_decay: float = 0.0, process_group=None, use_graphs: bool = True,
                  sinusoid: Optional[torch.Tensor] = None, lr_schedule: Optional[LRSchedule] = None,
                  max_grad_norm: Optional[float] = None, param_groups: Optional[Sequence[ParamGroup]] = None,
-                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None):
+                 optimizer: Optional[SGD] = None, param_stats: Optional[ParamStats] = None,
+                 weight_average: Optional[WeightAverage] = None):
         self.spec = spec
         self.device = torch.device(device)
         self.engine = TranslatorEngine(spec, self.device, dtype)
@@ -804,7 +908,8 @@ class TranslatorTrainer(_OptimizerState):
                 L.call("egot2_dropout_epoch_set", 0, torch.cuda.current_stream(self.device).cuda_stream)
         self._step_dev = torch.zeros(1, device=self.device, dtype=torch.int32)
         self._step_dev_val = 0
-        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats)
+        self._init_optimizer_state(lr_schedule, lr, 5e-4, max_grad_norm, param_groups, optimizer, param_stats,
+                                   weight_average)
         self._bump_stream = torch.cuda.Stream(device=self.device)
         self._peer_stream = torch.cuda.Stream(device=self.device)
         self._graphs: Dict[int, tuple] = {}
@@ -833,6 +938,7 @@ class TranslatorTrainer(_OptimizerState):
         graph on first use.  The captured kernels keep the dropout seed they were captured with; the device-resident
         dropout epoch (advanced once per step, folded into every key at execution time) makes each replay draw fresh
         masks all the same."""
+        self._check_training_weights()
         self.step_count += 1
         if self.dropout_epoch:
             self._epoch += 1               # every path below advances the device epoch once
@@ -939,16 +1045,18 @@ class TranslatorTrainer(_OptimizerState):
                 nb, n = self.engine.arena.embed_numel, self.engine.arena.numel
                 self._peer_stream.wait_stream(cur)
                 with torch.cuda.stream(self._peer_stream):
-                    self._peer_step(self._peer_stream.cuda_stream, step_dev=self._step_dev, lo=nb, hi=n, channel=0,
-                                    lr_dev=self._graph_lr_dev(), groups=self._groups)
+                    self._peer_step(self._peer_stream.cuda_stream, average=False, step_dev=self._step_dev, lo=nb, hi=n,
+                                    channel=0, lr_dev=self._graph_lr_dev(), groups=self._groups)
                 self.engine.backward(act, zero_grad=False, stage="embed")
                 self._bump_stream.wait_stream(cur)
                 with torch.cuda.stream(self._bump_stream):
                     self._advance_epoch()
-                self._peer_step(cur.cuda_stream, step_dev=self._step_dev, lo=0, hi=nb, channel=1,
+                self._peer_step(cur.cuda_stream, average=False, step_dev=self._step_dev, lo=0, hi=nb, channel=1,
                                 lr_dev=self._graph_lr_dev(), groups=self._groups)
                 cur.wait_stream(self._peer_stream)
                 cur.wait_stream(self._bump_stream)
+                if self._avg is not None:             # once, over the parameters both pieces gathered
+                    self._avg_launch(cur.cuda_stream)
                 self._grad_clean = True
                 self._graphs[key] = (g, act)
                 return g, act

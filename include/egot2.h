@@ -47,6 +47,8 @@
  *   egot2_param_stats            the add_histogram(name, weight) / add_histogram(name.grad, weight.grad) of the HOI LTA task's
  *                                gradient logging every LOG_GRADIENT_PERIOD steps (HOI/tasks/lta/video_task.py:112-125)
  *                                and Lightning's grad_norm, per parameter, on the device
+ *   egot2_weight_avg_update      torch.optim.swa_utils.AveragedModel's update_parameters over the flat arena: the EMA of
+ *                                get_ema_multi_avg_fn and the equal-weight SWA mean (Lightning's StochasticWeightAveraging)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer (row-major, contiguous) unless the name ends in _host;
@@ -574,6 +576,20 @@ int egot2_param_stats(const float* grad, const float* param, float grad_scale, c
                       egot2_param_stats_desc* desc, const egot2_stats_param* params, int32_t n_params,
                       const egot2_stats_unit* units, int32_t n_units, const double* edges, egot2_param_stat* stats,
                       int32_t* counts, void* workspace, size_t ws_bytes, void* stream);
+
+/* Weight averaging (torch.optim.swa_utils.AveragedModel) of the fp32 arena, after the optimizer launch of a step.  A step t
+ * (*step_dev, the applied-step count, read when the kernel executes) is due when t >= start and (t - start) % every == 0;
+ * on a due step, with n = (t - start) / every the number of earlier updates:
+ *   n == 0:  avg = param                                            (AveragedModel's first update_parameters copies)
+ *   n > 0:   avg = lerp(avg, param, w),  w = ema_weight (EGOT2_AVG_EMA: float(1 - decay), get_ema_multi_avg_fn)
+ *                                        w = 1 / (n + 1) in fp32     (EGOT2_AVG_SWA: the running mean; ema_weight unused)
+ * lerp is ATen's: w < 0.5 ? a + w * (p - a) : p - (p - a) * (1 - w), in fp32 with each product-and-sum fused into one FMA,
+ * as torch's CUDA _foreach_lerp_ rounds it.  guard (NULL: none): when guard->skip is set the step was skipped and nothing
+ * changes, whatever *step_dev holds.  On a step that is not due every CTA returns at once.  n is a multiple of 4 and both
+ * arrays are 16-byte aligned.  No host sync; graph-capturable. */
+enum { EGOT2_AVG_EMA = 0, EGOT2_AVG_SWA = 1 };
+int egot2_weight_avg_update(const float* param, float* avg, size_t n, int32_t kind, float ema_weight, int32_t every,
+                            int32_t start, const int32_t* step_dev, const egot2_grad_guard* guard, void* stream);
 
 /* ------------------------------------------------------------------ data-parallel exchange over NVLink peer memory
  * The reference trains under DDP / DP (HOI/scripts/lta/run_lta.py:249, HOI/tasks/pnr/video_task.py:39-42): an all-reduce of the
